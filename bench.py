@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- EOT-samples/sec of the DorPatch hot loop (BASELINE.json metric).
 
-    python bench.py [--gpus N --steps K --warmup W] [--impl native|reference] [--precision tf32|bf16|fp32]
+    python bench.py [--gpus N --steps K --warmup W] [--impl native|reference] [--precision tf32|bf16|fp32] [--dump-outputs DIR]
 
 A "step" is one iteration of attack.py:184-342 of the reference over one batch: sample occlusion masks on the host,
 paste + expand (K1), ResNetV2-50x1-BiT forward + backward-to-input (K2), CW loss (K4), masked EOT gradient reduce
@@ -26,6 +26,13 @@ input carries a zero pad channel for the library stem), `traffic` the DRAM bytes
 ("c5": targeted, 10 % budget, density + group-lasso regularisers live), PatchCleanser evaluation throughput, and the
 scan-amortised throughput (the reference re-scans the whole mask universe every 100 steps, attack.py:187-190); the c3 / c2
 legs carry the K1 roofline of their own launch shape (`k1_roofline`).  `--config c5s0 --gpus 4` = configs[4] on 4 GPUs.
+Every timed run (headline, e2e, each leg) is K steps.
+
+`--dump-outputs DIR` writes, after the headline's timed steps, what its last step handed back to the caller as DIR/<name>.npy
+(float32): attack_grad's host results (loss_adv, preds, loss_struc, loss_density, group_lasso, l2), the patch gradient
+grad_adv and the mask / pattern after the sign step.  An array of more than DUMP_MAX_ELEMENTS elements is written as the
+same seeded sample of that many of its flattened elements (sorted indices), so the dump stays under 64 MB.  The inputs are
+seeded, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -44,6 +51,7 @@ IMG = 224
 SAMPLES_PER_GPU = 2048           # c3: 64 x 32
 GFLOP_PER_SAMPLE = 16.36         # 8.18 fwd + 8.18 dgrad (SURVEY.md section 8d)
 METRIC, UNIT = "EOT-samples/sec", "samples/s"
+DUMP_MAX_ELEMENTS = 1 << 22
 CONFIGS = {   # name -> (images, EOT per image [total], stage, targeted, budget)
     "c3": dict(B=64, S=32, stage=1, targeted=False, budget=0.12),
     "c2": dict(B=32, S=16, stage=1, targeted=False, budget=0.05),
@@ -144,6 +152,19 @@ def cpu_step_factory(S):
         state["pattern"] = (state["pattern"] - 0.01 * r["grad_pattern"].sign()).clamp(0, 1)
         return S
     return step, torch.get_num_threads()
+
+
+def dump_outputs(arrays, out_dir):
+    """arrays: name -> host array; written as float32 .npy files, larger ones as a fixed seeded sample (module docstring)."""
+    os.makedirs(out_dir, exist_ok=True)
+    total = 0
+    for name, a in arrays.items():
+        a = np.ascontiguousarray(a, np.float32)
+        if a.size > DUMP_MAX_ELEMENTS:
+            a = a.reshape(-1)[np.sort(np.random.default_rng(0).choice(a.size, DUMP_MAX_ELEMENTS, replace=False))]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+        total += a.nbytes
+    assert total <= 64 << 20, total
 
 
 def workload_config(config, world, precision=None):
@@ -265,6 +286,13 @@ class Workload:
         lr, st_used, cg_used = self.finish(i, idx, r, self.G)
         self.host_s += time.perf_counter() - t0               # exchange + bookkeeping (the all-reduce runs under it)
         self.eng.attack_update(self.x, self.mask, self.pattern, self.G, lr, st_used, cg_used, 1e-3, self.stage)
+        self.last = r
+
+    def outputs(self):
+        """What the last step() handed back: attack_grad's host results, the patch gradient, the updated mask / pattern."""
+        out = {k: np.asarray(v, np.float32) for k, v in self.last.items()}
+        out.update(grad_adv=self.G.cpu().numpy(), mask=self.mask.cpu().numpy(), pattern=self.pattern.cpu().numpy())
+        return out
 
     def step_e2e(self, i):
         import torch
@@ -350,7 +378,7 @@ def run_native(args):
 
     W, K = max(args.warmup, 3), args.steps
 
-    def measure(precision, config, K, e2e=True, sampler=None):
+    def measure(precision, config, K, e2e=True, sampler=None, keep_outputs=False):
         eng = engine(precision)
         wl = Workload(eng, config, world, rank, dev, dist if world > 1 else None)
         for i in range(W):
@@ -361,7 +389,8 @@ def run_native(args):
         wl.host_s = 0.0
         ms, launches = timed(eng, wl.step, K, W)
         clocks = sampler.stop() if sampler is not None else None
-        res = dict(value=wl.samples_per_step * K / (ms / 1e3), ms_per_step=ms / K, launches=int(launches), clocks=clocks, wl=wl, eng=eng,
+        outputs = wl.outputs() if keep_outputs else None
+        res = dict(outputs=outputs, value=wl.samples_per_step * K / (ms / 1e3), ms_per_step=ms / K, launches=int(launches), clocks=clocks, wl=wl, eng=eng,
                    host_ms=wl.host_s / K * 1e3, graph_replays=eng.graph_replays)
         if e2e:
             for i in range(2):
@@ -383,7 +412,9 @@ def run_native(args):
         torch.cuda.profiler.stop()
         return
 
-    head = measure(args.precision, args.config, K, e2e=True, sampler=ClockSampler(local))
+    head = measure(args.precision, args.config, K, e2e=True, sampler=ClockSampler(local), keep_outputs=bool(args.dump_outputs))
+    if args.dump_outputs and rank == 0:
+        dump_outputs(head.pop("outputs"), args.dump_outputs)
     wl, eng = head["wl"], head["eng"]
     h2d, d2h = wl.io_bytes()
     out = {
@@ -568,17 +599,16 @@ def run_native(args):
             out.setdefault("scan", {"error": str(ex)[:300]})
             out["patchcleanser_eval"] = {"error": str(ex)[:300]}
     del wl
-    # ---- extra legs (single GPU only; each is a full timed run of K2 steps) ----------------------------------------------
+    # ---- extra legs (single GPU only; each is a full timed run of K steps) -----------------------------------------------
     if world == 1 and not args.no_legs:
         legs = {}
-        K2 = max(3, min(K, 10))
         other = "bf16" if args.precision != "bf16" else "tf32"
         plan = [(args.precision, "c2"), (args.precision, "b1"), (args.precision, "c5s0"), (other, "c3"), (other, "c2"), (other, "b1")]
         for prec, cfg in plan:
             if cfg == args.config and prec == args.precision:
                 continue
             try:
-                r = measure(prec, cfg, K2 if cfg != "b1" else 20, e2e=(cfg in ("c2", "c3")))
+                r = measure(prec, cfg, K, e2e=(cfg in ("c2", "c3")))
                 leg = {"value": r["value"], "ms_per_step": r["ms_per_step"], "gpu_launches": r["launches"], "dtype": prec, "host_ms_per_step": r["host_ms"],
                        "config": workload_config(cfg, 1)["workload"]}
                 if "e2e_value" in r:
@@ -631,7 +661,10 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-legs", action="store_true", help="skip the extra legs (bf16 / c2 / B=1 / stage 0)")
     ap.add_argument("--ncu", action="store_true", help="run W warm-up steps, then ONE step inside cudaProfilerStart/Stop, and exit")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs to DIR/<name>.npy (see the module docstring)")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "native" or args.ncu):
+        ap.error("--dump-outputs dumps the native arm's timed steps: it needs --impl native and no --ncu")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -1,10 +1,8 @@
-"""Import the UNMODIFIED reference (/root/reference) on a CPU-only box.
+"""Import the UNMODIFIED reference (a checkout of CGCL-codes/DorPatch) on a CPU-only box.
 
-Used only in the build container (``/root/reference`` does not exist on the GPU
-box) by ``tests/golden/make_golden.py`` to generate golden vectors and by
-``tests/test_oracle_vs_reference.py`` (skipped when the reference is absent) to
-pin the oracle.  Nothing is copied: the reference modules are imported from
-where they lie.
+Used only by ``tests/golden/make_golden.py`` to generate the golden vectors the
+test suite pins the oracle against; the suite itself never needs the reference.
+Nothing is copied: the reference modules are imported from where they lie.
 
 Shim (SURVEY.md section 8c):
   * ``Tensor.cuda`` / ``Tensor.cpu`` return a *copy* on the CPU (on a GPU box
@@ -14,7 +12,7 @@ Shim (SURVEY.md section 8c):
     ``Module.cuda`` is identity;
   * ``timm`` (not installed, third-party) is replaced by an empty stub module --
     ``utils.get_model`` is never called, the caller passes its own model;
-  * ``/root/reference`` is put on ``sys.path`` so ``attack``, ``utils`` and
+  * the reference checkout is put on ``sys.path`` so ``attack``, ``utils`` and
     ``defenses.PatchCleanser`` resolve to the reference's files.
 TEST INFRASTRUCTURE ONLY (see oracle/__init__.py).
 """
@@ -25,16 +23,15 @@ import os
 import sys
 import types
 
-REFERENCE_ROOT = "/root/reference"
 _REF_MODULES = ("attack", "utils", "defenses", "defenses.PatchCleanser", "main")
 
 
-def available():
-    return os.path.isfile(os.path.join(REFERENCE_ROOT, "attack.py"))
+def available(root):
+    return os.path.isfile(os.path.join(root, "attack.py"))
 
 
 @contextlib.contextmanager
-def reference_modules():
+def reference_modules(root):
     """Context manager yielding a namespace with the reference's ``attack``,
     ``utils`` and ``PatchCleanser`` modules; restores sys.modules/sys.path and
     the torch monkeypatches on exit so the product's same-named root modules
@@ -48,7 +45,7 @@ def reference_modules():
         for k in _REF_MODULES:
             sys.modules.pop(k, None)
         sys.modules["timm"] = types.ModuleType("timm")
-        sys.path.insert(0, REFERENCE_ROOT)
+        sys.path.insert(0, root)
         torch.Tensor.cuda = lambda self, *a, **k: self.clone()
         torch.Tensor.cpu = lambda self, *a, **k: self.clone()
         torch.nn.Module.cuda = lambda self, *a, **k: self
@@ -56,11 +53,11 @@ def reference_modules():
         # Load by file path: the repo root holds same-named drop-in modules (attack, utils,
         # defenses/ -- a regular package, which would shadow the reference's namespace package).
         pkg = types.ModuleType("defenses")
-        pkg.__path__ = [os.path.join(REFERENCE_ROOT, "defenses")]
+        pkg.__path__ = [os.path.join(root, "defenses")]
         sys.modules["defenses"] = pkg
 
         def load(name, rel):
-            spec = importlib.util.spec_from_file_location(name, os.path.join(REFERENCE_ROOT, rel))
+            spec = importlib.util.spec_from_file_location(name, os.path.join(root, rel))
             mod = importlib.util.module_from_spec(spec)
             sys.modules[name] = mod
             spec.loader.exec_module(mod)
@@ -69,7 +66,7 @@ def reference_modules():
         ns.utils = load("utils", "utils.py")
         ns.PatchCleanser = load("defenses.PatchCleanser", "defenses/PatchCleanser.py")
         ns.attack = load("attack", "attack.py")
-        assert ns.attack.__file__.startswith(REFERENCE_ROOT), ns.attack.__file__
+        assert ns.attack.__file__.startswith(root), ns.attack.__file__
         assert ns.attack.MaskWindow is ns.PatchCleanser.MaskWindow and ns.attack.clip is ns.utils.clip
         yield ns
     finally:

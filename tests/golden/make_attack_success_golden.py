@@ -15,6 +15,8 @@ eps 4), adv_x = x + clip(mask, pattern, x, eps) (main.py:140-141), robust_predic
 for ratios 0.015/0.03/0.06/0.12 (main.py:61,151), model(adv_x).argmax (main.py:156).
 tests/test_gpu_attack_success.py replays the same protocol on the native engine (fp32 / tf32 /
 bf16) and compares the bits and the main.py:162-185 rates.  Output: attack_success_golden.npz.
+The final adversarial images are stored as adv_delta = adv_x - x_i (x_i unperturbed), which is
+mostly zero and compresses; image(i) + adv_delta[i] reproduces adv_x bit for bit (asserted).
 """
 import os
 import random
@@ -61,7 +63,7 @@ def main():
     torch.set_num_threads(min(16, os.cpu_count() or 1))
     params = OR.random_init(seed=0, affine_jitter=0.1)
     net = OR.OracleNet(params, weights_require_grad=False).eval()
-    rec = dict(y=[], pred_adv=[], pc_pred=[], pc_cert=[], mask_frac=[], l2=[], steps=[], adv=[], margin=[])
+    rec = dict(y=[], pred_adv=[], pc_pred=[], pc_cert=[], mask_frac=[], l2=[], steps=[], adv_delta=[], margin=[])
     t0 = time.time()
     for i in range(K):
         x = image(i)
@@ -87,7 +89,9 @@ def main():
         rec["mask_frac"].append(float(m.mean())); rec["l2"].append(float(delta.norm())); rec["steps"].append(len(trace))
         rec["margin"].append(float(top2[0] - top2[1]))
         if a.save_adv:
-            rec["adv"].append(adv[0].numpy().copy())
+            d = adv[0].numpy() - image(i)[0].numpy()
+            assert np.array_equal(image(i)[0].numpy() + d, adv[0].numpy())
+            rec["adv_delta"].append(d)
         print("img %2d  y %3d  adv %3d (top-2 margin %.2e)  PC %s cert %s  mask %.4f  l2 %.3f  steps %d  (%.0f s)" % (
             i, y, pa, rec["margin"][-1], preds, [int(c) for c in certs], rec["mask_frac"][-1], rec["l2"][-1], len(trace), time.time() - t0),
             flush=True)

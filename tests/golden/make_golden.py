@@ -1,13 +1,15 @@
-"""Generate golden vectors by running the UNMODIFIED reference (/root/reference) under the CPU
-shim of oracle/ref_shim.py.  Run in the build container only (the reference is absent on
-the GPU box); the resulting small .npz fixtures are committed next to this script.
+"""Generate golden vectors by running the UNMODIFIED reference (a checkout of
+CGCL-codes/DorPatch @ 0751fd4) under the CPU shim of oracle/ref_shim.py.  The resulting .npz
+fixture is committed next to this script, so the test suite never needs the reference.
 
-    python tests/golden/make_golden.py
+    python tests/golden/make_golden.py --reference <path of the reference checkout>
 
 Pins (SURVEY.md section 4): G1 mask geometry, G2 utils.clip, G3 losses + gradients,
 G4 patch_selection, G5/G6 generate trajectories (tiny stand-in classifier: targeted 10 steps,
 and untargeted 1100 steps crossing the i==500 targeted switch, the i>=1000 failed-set sampling
-and the lr-decay path), G7 PatchCleanser records, G9 a ResNetV2-50 trajectory at 112 px.
+and the lr-decay path), G7 PatchCleanser records, G9 a ResNetV2-50 trajectory at 112 px,
+G10 a 25-step targeted dropout-2 trajectory (tiny classifier, absolute target label).
+The G2 inputs are not stored: g2_inputs() re-draws them from their seed.
 """
 import contextlib
 import io
@@ -48,6 +50,25 @@ def seed_all(s=1234):
     np.random.seed(s)
 
 
+def g2_inputs():
+    """The seeded inputs of G2 (image, mask, pattern, output weights) and the generator, which G3 and G4 draw on from there."""
+    g = torch.Generator().manual_seed(11)
+    x = torch.rand(3, 3, 56, 56, generator=g)
+    m = torch.rand(3, 1, 56, 56, generator=g)
+    p = torch.rand(3, 3, 56, 56, generator=g)
+    m[1] *= 0.01
+    w = torch.rand(3, 3, 56, 56, generator=g)
+    return g, x, m, p, w
+
+
+G10_KW = dict(patch_budget=0.12, n_classes=1000, targeted=True, y=torch.tensor([7]), max_iterations=25, sampling_size=3,
+              dropout=2)
+
+
+def g10_input():
+    return torch.rand(1, 3, 56, 56, generator=torch.Generator().manual_seed(21))
+
+
 def run_generate(ref, net, x, **kw):
     """Reference generate in a scratch cwd (it writes stage-0 artefacts relative to cwd)."""
     cwd = os.getcwd()
@@ -69,10 +90,14 @@ def run_generate(ref, net, x, **kw):
 
 
 def main():
-    assert ref_shim.available(), "reference not present"
+    import argparse
+    ap = argparse.ArgumentParser()
+    ap.add_argument("--reference", required=True, help="checkout of the unmodified reference (CGCL-codes/DorPatch @ 0751fd4)")
+    root = os.path.abspath(ap.parse_args().reference)
+    assert ref_shim.available(root), "no reference at %s" % root
     torch.set_num_threads(8)
     out = {}
-    with ref_shim.reference_modules() as ref:
+    with ref_shim.reference_modules(root) as ref:
         A, U, PC = ref.attack, ref.utils, ref.PatchCleanser
         # ---- G1 geometry -----------------------------------------------------------------
         with contextlib.redirect_stdout(io.StringIO()):
@@ -85,17 +110,11 @@ def main():
                     out["g1_double_sum_%d_%s" % (H, r)] = dm.reshape(dm.shape[0], -1).sum(1).astype(np.int32)
                     out["g1_double_probe_%d_%s" % (H, r)] = np.packbits(dm[[0, 1, 35, 36, 300, 629]])
         # ---- G2 clip -----------------------------------------------------------------------
-        g = torch.Generator().manual_seed(11)
-        x = torch.rand(3, 3, 56, 56, generator=g)
-        m = torch.rand(3, 1, 56, 56, generator=g)
-        p = torch.rand(3, 3, 56, 56, generator=g)
-        m[1] *= 0.01
+        g, x, m, p, w = g2_inputs()
         mm, pp = m.clone().requires_grad_(True), p.clone().requires_grad_(True)
         d = U.clip(mm, pp, x, 4.0)
-        w = torch.rand(d.shape, generator=g)
         (d * w).sum().backward()
-        out.update(g2_x=x.numpy(), g2_m=m.numpy(), g2_p=p.numpy(), g2_w=w.numpy(), g2_delta=d.detach().numpy(),
-                   g2_gm=mm.grad.numpy(), g2_gp=pp.grad.numpy())
+        out.update(g2_delta=d.detach().numpy(), g2_gm=mm.grad.numpy(), g2_gp=pp.grad.numpy())
         # ---- G3 losses + gradients ------------------------------------------------------------
         xa = torch.rand(2, 3, 56, 56, generator=g).requires_grad_(True)
         lv, lr_, ud = A.local_variance(xa)
@@ -104,7 +123,7 @@ def main():
         ls = torch.mean(mv.mean(1) / (lvx + 1e-5), (1, 2))
         ls.sum().backward()
         out.update(g3_x=xa.detach().numpy(), g3_lv=lv.detach().numpy(), g3_mv=mv.detach().numpy(),
-                   g3_ls=ls.detach().numpy(), g3_ls_grad=xa.grad.numpy(), g3_lvx_src=x[:2].numpy())
+                   g3_ls=ls.detach().numpy(), g3_ls_grad=xa.grad.numpy())
         ma = torch.rand(2, 1, 56, 56, generator=g)
         ma[0, 0, :7, 7:14] = 0
         ma = ma.requires_grad_(True)
@@ -181,6 +200,9 @@ def main():
         out["g9_log"] = np.array(log)
         out["g9_rng_np"] = rn
         out["g9_target"] = ((yr + 17) % 1000).numpy()
+        # ---- G10 a dropout-2 trajectory with an absolute target label (tiny classifier) ----------------------------
+        mo, po, log, rn, rt = run_generate(ref, tiny, g10_input(), **G10_KW)
+        out.update(g10_mask=mo, g10_pattern=po, g10_log=np.array(log), g10_rng_np=rn)
     np.savez_compressed(os.path.join(HERE, "reference_golden.npz"), **out)
     print("wrote", os.path.join(HERE, "reference_golden.npz"), os.path.getsize(os.path.join(HERE, "reference_golden.npz")))
 

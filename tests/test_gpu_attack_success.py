@@ -118,13 +118,14 @@ def _report(tag, precision, y, g, pred_adv, pc_pred, pc_cert):
 @pytest.mark.parametrize("precision", PRECISIONS)
 def test_evaluation_bits_on_frozen_adversarial_images(oracle_params, precision):
     g = _load(GOLD)
-    if "adv" not in g.files:
+    if "adv_delta" not in g.files:
         pytest.skip("attack_success_golden.npz holds no adversarial images: regenerate it (--save-adv 1)")
     K, img = int(g["K"]), int(g["img"])
     y = g["y"].astype(np.int64)
+    adv = torch.cat([_image(i, img, g["img_seed0"]) for i in range(K)]) + torch.from_numpy(g["adv_delta"])
     pipe = _Pipeline(oracle_params, precision, img, K, g["ratios"])
     try:
-        pred_adv, pc_pred, pc_cert = pipe.evaluate(torch.from_numpy(g["adv"]).to(DEV))
+        pred_adv, pc_pred, pc_cert = pipe.evaluate(adv.to(DEV))
     finally:
         pipe.close()
     _report("frozen", precision, y, g, pred_adv, pc_pred, pc_cert)

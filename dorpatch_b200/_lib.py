@@ -8,7 +8,7 @@ import os
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "lib", "libdorpatch.so")
-ABI_VERSION = 6
+ABI_VERSION = 7
 
 c_i32, c_i64, c_f32, c_vp = C.c_int32, C.c_int64, C.c_float, C.c_void_p
 
@@ -66,7 +66,8 @@ SIGNATURES = {
     "dp_failed_set_write": (c_i32, [c_vp, c_i32, c_vp, c_i32, c_vp]),
     "dp_failed_set_update": (c_i32, [c_vp, c_i32, c_i32, c_vp, c_vp, c_vp, c_vp, c_f32, c_vp, c_vp]),
     "dp_failed_set_read": (c_i32, [c_vp, c_i32, c_vp, c_i32, c_vp, c_vp]),
-    "dp_debug_stem_bwd_reduce": (c_i32, [c_vp, c_vp, c_vp, c_i32, c_i32, c_vp, c_vp]),
+    "dp_debug_k1t": (c_i32, [c_vp, c_vp, c_vp, c_i32, c_i32, c_i32, c_i32, c_vp, c_vp]),
+    "dp_debug_cw": (c_i32, [c_vp, c_vp, c_vp, c_vp, c_f32, c_f32, c_vp, c_vp, c_vp, c_i32, c_i32, c_vp]),
     "dp_debug_gn_gemm": (c_i32, [c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_i32, c_i32, c_i32, c_i32, c_vp]),
     "dp_debug_gn": (c_i32, [c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_i32, c_vp, c_vp, c_vp, c_i32, c_i32, c_i32, c_vp]),
 }

@@ -1413,18 +1413,33 @@ int32_t dp_failed_set_read(dp_engine* e, int32_t b, int32_t* idx_host_out, int32
   DP_CATCH
 }
 
-/* ---- op-level test hooks (tests/test_gpu_ops.py) ------------------------------------------------------ */
-int32_t dp_debug_stem_bwd_reduce(dp_engine* e, const void* dY, const int16_t* rects_host, int32_t B, int32_t S, float* G,
-                                 void* stream) {
+/* ---- op-level test hooks (tests/test_gpu_ops.py, tests/test_gpu_patch_kernels.py) --------------------- */
+int32_t dp_debug_k1t(dp_engine* e, const void* dz, const int16_t* rects_host, int32_t B, int32_t S, int32_t n0, int32_t n,
+                     float* G, void* stream) {
   DP_TRY
   if (!e) fail("null engine");
-  if (!e->own_stem) fail("dp_debug_stem_bwd_reduce: the fused stem backward exists for the bf16 engine only");
+  if (!dz || !G) fail("dp_debug_k1t: null pointer");
+  if (B < 1 || S < 1 || n0 < 0 || n < 1 || n0 + n > B * S) fail("dp_debug_k1t: samples [%d, %d) outside [0, %d)", n0, n0 + n, B * S);
   CUDA_OK(cudaSetDevice(e->cfg.device));
   cudaStream_t st = (cudaStream_t)stream;
-  const int N = B * S;
-  e->h2d_samples(rects_host, N, st);
-  CUDA_OK(cudaMemsetAsync(G, 0, (size_t)B * 3 * e->H * e->H * 4, st));
-  dp::launch_stem_bwd_reduce(dY, e->stem.w, e->stem.cin_pad, rects_host ? e->rects_d : nullptr, G, B, S, 0, N, e->H, e->H, st);
+  e->h2d_samples(rects_host, B * S, st);
+  const int16_t* rects = rects_host ? e->rects_d : nullptr;
+  // the K1^T of dp_attack_grad's chunk loop for this engine (G is not cleared: the first launch of an image overwrites it)
+  if (e->stem_bwd_fused_ok()) dp::launch_stem_bwd_reduce(dz, e->stem.w, e->stem.cin_pad, rects, G, B, S, n0, n, e->H, e->H, st);
+  else dp::launch_reduce(dz, rects, G, B, S, n0, n, e->H, e->H, e->Cpd, e->bf16, st);
+  KERNEL_OK(); ++e->launches;
+  DP_CATCH
+}
+
+int32_t dp_debug_cw(dp_engine* e, const float* logits, const int32_t* y, const uint8_t* targeted, float confidence, float w,
+                    float* loss, int32_t* preds, float* dlogits, int32_t N, int32_t K, void* stream) {
+  DP_TRY
+  if (!e) fail("null engine");
+  if (!logits || N < 1 || K < 1) fail("dp_debug_cw: bad arguments");
+  if (loss && (!y || !targeted)) fail("dp_debug_cw: the loss needs labels and criterion flags");
+  CUDA_OK(cudaSetDevice(e->cfg.device));
+  cudaStream_t st = (cudaStream_t)stream;
+  dp::launch_cw(logits, y, targeted, confidence, w, loss, preds, dlogits, N, K, st);
   KERNEL_OK(); ++e->launches;
   DP_CATCH
 }

@@ -489,6 +489,14 @@ void launch_reduce_affine(const void* dz, const float* adv, const float* xf, con
 // =====================================================================================
 // K4: CW loss / argmax / dlogits -- one warp per sample
 // =====================================================================================
+// Does logit (v, i) come before the current pick (best, bi)?  torch.argmax / torch.max order: a NaN ranks above every
+// number (the first NaN wins), equal values go to the lower index.
+__device__ __forceinline__ bool cw_before(float v, int i, float best, int bi) {
+  const bool vn = v != v, bn = best != best;
+  if (vn != bn) return vn;
+  if (!vn && v != best) return v > best;
+  return i < bi;
+}
 __global__ void cw_kernel(const float* __restrict__ logits, const int32_t* __restrict__ y,
                           const uint8_t* __restrict__ targeted, float confidence, float w, float* __restrict__ loss,
                           int32_t* __restrict__ preds, float* __restrict__ dlogits, int N, int K) {
@@ -497,28 +505,33 @@ __global__ void cw_kernel(const float* __restrict__ logits, const int32_t* __res
   const float* l = logits + (size_t)n * K;
   const int yy = y != nullptr ? y[n] : -1;
   float best = -INFINITY, obest = -INFINITY; int bi = 0x7fffffff, oi = 0x7fffffff;
+  bool finite = true;
   for (int k = lane; k < K; k += 32) {
     const float v = l[k];
-    if (v > best) { best = v; bi = k; }
-    if (k != yy && v > obest) { obest = v; oi = k; }
+    finite = finite && isfinite(v);
+    if (cw_before(v, k, best, bi)) { best = v; bi = k; }
+    if (k != yy && cw_before(v, k, obest, oi)) { obest = v; oi = k; }
   }
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) {
     const float v2 = __shfl_xor_sync(0xffffffffu, best, o); const int i2 = __shfl_xor_sync(0xffffffffu, bi, o);
-    if (v2 > best || (v2 == best && i2 < bi)) { best = v2; bi = i2; }
+    if (cw_before(v2, i2, best, bi)) { best = v2; bi = i2; }
     const float w2 = __shfl_xor_sync(0xffffffffu, obest, o); const int j2 = __shfl_xor_sync(0xffffffffu, oi, o);
-    if (w2 > obest || (w2 == obest && j2 < oi)) { obest = w2; oi = j2; }
+    if (cw_before(w2, j2, obest, oi)) { obest = w2; oi = j2; }
   }
   if (lane == 0 && preds != nullptr) preds[n] = bi;
   if (loss == nullptr) return;
+  finite = __all_sync(0xffffffffu, finite);
   const float real = l[yy];
-  // attack.py:19: the label slot contributes -1e4 to the max
-  const bool other_is_label_slot = !(obest > -1e4f);
+  // attack.py:19: the label slot contributes -1e4 to the max (and wins a tie at -1e4 when its index is the lower one)
+  const bool other_is_label_slot = obest < -1e4f || (obest == -1e4f && yy < oi);
   const float other = other_is_label_slot ? -1e4f : obest;
   const bool tg = targeted[n] != 0;
   const float margin = tg ? (other - real) : (real - other);
-  const float pre = confidence + margin;
-  if (lane == 0) loss[n] = fmaxf(pre, 0.f);
+  // attack.py:18-19 multiply the logits by the one-hot label: one non-finite logit (0 * inf = NaN) makes the loss NaN,
+  // which torch.clamp passes on (a failed sample) with a zero gradient
+  const float pre = finite ? confidence + margin : NAN;
+  if (lane == 0) loss[n] = isnan(pre) ? pre : fmaxf(pre, 0.f);
   if (dlogits != nullptr) {
     float* d = dlogits + (size_t)n * K;
     for (int k = lane; k < K; k += 32) d[k] = 0.f;

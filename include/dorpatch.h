@@ -35,7 +35,7 @@
 extern "C" {
 #endif
 
-#define DP_ABI_VERSION 6
+#define DP_ABI_VERSION 7
 
 enum dp_precision {
   DP_PREC_FP32 = 0, /* fp32 storage, fp32 FMA math (no tensor cores): parity checks   */
@@ -112,7 +112,8 @@ int32_t dp_expand(dp_engine* e, const float* img, int32_t B, int32_t S, const in
 int32_t dp_expand_dev(dp_engine* e, const float* img, int32_t B, int32_t S, const int16_t* rects_dev,
                       void* out, void* stream);
 /* The variant of K1 the hot loop launches (attack.py:184-185 fused in: reads x / mask / pattern [B,...] dev and the
- * clip scale of the last dp_paste / dp_attack_grad on these tensors), for samples [n0, n0+n) of the b-major
+ * engine's per-image clip scale, which only the last dp_attack_grad or dp_paste with adv_x_out == NULL writes; a
+ * dp_paste with an output buffer leaves it alone), for samples [n0, n0+n) of the b-major
  * [B*S] ordering -- one classifier chunk.  Rectangles on the device; exactly one kernel launch, no synchronisation
  * (bench.py's roofline leg times this launch). */
 int32_t dp_expand_step_dev(dp_engine* e, const float* x, const float* mask, const float* pattern, int32_t B, int32_t S,
@@ -208,16 +209,25 @@ int32_t dp_failed_set_update(dp_engine* e, int32_t B, int32_t S, const int32_t* 
                              void* stream);
 int32_t dp_failed_set_read(dp_engine* e, int32_t b, int32_t* idx_host_out, int32_t cap, int32_t* n_out, void* stream);
 
-/* Op-level hooks for the parity tests (tests/test_gpu_ops.py); not part of the reference-facing surface.
- * dp_debug_stem_bwd_reduce: the bf16 engine's fused stem-dgrad + masked EOT reduce (K1^T as the bench runs it) on a
- *   caller-supplied dY [B*S, H/2, H/2, 64] bf16 dev: G[B,3,H,W] = 2 * sum_s keep_s * conv7x7s2^T(dY_s, W_stem).
+/* Op-level hooks for the parity tests (tests/test_gpu_ops.py, tests/test_gpu_patch_kernels.py); not part of the
+ * reference-facing surface.
+ * dp_debug_k1t: the K1^T dp_attack_grad runs for samples [n0, n0+n) of the b-major [B*S] ordering, into the caller's
+ *   G [B,3,H,W] fp32 dev: G[b] = 2 * sum_s keep_s * dX_s over the launch's samples of image b, OVERWRITING G[b] when the
+ *   launch holds image b's first sample and adding to it otherwise (G is not cleared).  rects_host as in dp_expand.
+ *   dz is the chunk's slice (sample n0 first): on the bf16 engine with the fused stem backward dz = dY
+ *   [n, H/2, W/2, 64] bf16 and dX_s = conv7x7s2^T(dY_s, W_stem); otherwise dz = dX [n, H, W, Cpd] in the activation
+ *   dtype (Cpd = 4 fp32 / 8 bf16; channels >= 3 are ignored).
+ * dp_debug_cw: K4 on caller-supplied device buffers: logits [N,K] fp32, y [N] int32, targeted [N] uint8; writes
+ *   loss [N], preds [N] int32 and dlogits [N,K] (= w * d loss / d logits) -- each may be NULL (loss NULL: preds only).
  * dp_debug_gn_gemm: the tcgen05 GroupNorm-prologue GEMM on caller-supplied operands: out[m,n] = sum_k
  *   relu(gn(x))[m,k] * W[n,k] (+ shortcut); x [N*P,K] bf16, w_nk [Nout,K] bf16, stats [N,32,2] (mean, rstd), all dev.
  * dp_debug_gn: GroupNorm(32)+ReLU forward (and, with dy, backward-to-input) in the engine's activation dtype on
  *   caller-supplied [N,P,C] tensors; stats [N,32,2] dev out.  y == NULL: statistics pass only (the streaming
  *   kernel in front of the tcgen05 GEMM and the classifier head). */
-int32_t dp_debug_stem_bwd_reduce(dp_engine* e, const void* dY, const int16_t* rects_host, int32_t B, int32_t S, float* G,
-                                 void* stream);
+int32_t dp_debug_k1t(dp_engine* e, const void* dz, const int16_t* rects_host, int32_t B, int32_t S, int32_t n0, int32_t n,
+                     float* G, void* stream);
+int32_t dp_debug_cw(dp_engine* e, const float* logits, const int32_t* y, const uint8_t* targeted, float confidence, float w,
+                    float* loss, int32_t* preds, float* dlogits, int32_t N, int32_t K, void* stream);
 /* K1 launch-shape sweep hook (tools/k1_step_sweep.py): tile rows / sample groups (0 = the wave-efficiency heuristic) and the
  * store path (0 = bulk stores + 16-byte stores for occluded rows, 1 = 16-byte stores only).  Process-wide. */
 int32_t dp_debug_k1_tuning(int32_t rows, int32_t sg, int32_t mode);

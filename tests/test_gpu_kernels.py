@@ -323,29 +323,48 @@ def test_bf16_fused_stem_backward_reduce_matches_library_path(oracle_params):
     assert cos >= 0.9999 and rel <= 1e-2, (cos, rel)
 
 
+# engine option (read at create) -> (its two settings, B, S): results must not depend on it
+ENGINE_OPTIONS = {
+    # dp_attack_grad alternates chunks between two workspaces / streams when every chunk holds whole images
+    # (chunk 4, S 4: 3 chunks of one image each on lanes 0, 1, 0)
+    "DORPATCH_LANES": (("1", "2"), 3, 4),
+    # K1 per classifier chunk (0: launches [n0, n0+4) that split the 3-sample images) against one whole-step launch
+    "DORPATCH_K1_WHOLE_MB": (("0", None), 3, 3),
+}
+
+
+@pytest.mark.parametrize("option", list(ENGINE_OPTIONS))
 @pytest.mark.parametrize("precision", ["fp32", "bf16"])
-def test_two_lane_chunk_overlap_is_bit_identical(oracle_params, precision):
-    """dp_attack_grad alternates chunks between two workspaces / streams when every chunk holds whole images.
-    Same kernels, same inputs, disjoint outputs: the result must equal the single-lane run bit for bit."""
+def test_engine_option_does_not_change_results(oracle_params, precision, option):
+    """Same kernels, same inputs, a different schedule: one dp_attack_grad step must give the same patch gradient,
+    per-sample losses and predictions bit for bit under either setting of the option (None = unset, the default)."""
     import os
     from dorpatch_b200.engine import Engine
-    H, B, S = 112, 3, 4                       # chunk 4 -> 3 chunks, one image each, lanes 0,1,0
+    settings, B, S = ENGINE_OPTIONS[option]
+    H = 112
     x, m, p = _rand((B, 3, H, H), 81), _rand((B, 1, H, H), 82), _rand((B, 3, H, H), 83)
     rects = _rects_for(H, np.random.RandomState(6).randint(0, 2520, (B, S)), 2)
     y = np.array([1, 2, 3])
     out = {}
-    for lanes in ("1", "2"):
-        os.environ["DORPATCH_LANES"] = lanes
-        e = Engine(img=H, precision=precision, chunk=4, max_images=B, autotune=False)
+    for value in settings:
+        if value is None:
+            os.environ.pop(option, None)
+        else:
+            os.environ[option] = value
+        try:
+            e = Engine(img=H, precision=precision, chunk=4, max_images=B, autotune=False)
+        finally:
+            os.environ.pop(option, None)
         e.load_state_dict(oracle_params)
-        G = torch.zeros(B, 3, H, H, device=DEV)
+        G = torch.full((B, 3, H, H), float("nan"), device=DEV)
         r = e.attack_grad(x.to(DEV), m.to(DEV), p.to(DEV), rects, y, [True, False, True], 0.1, 4.0, 0, G)
         torch.cuda.synchronize()
-        out[lanes] = (G.cpu().clone(), r["loss_adv"].copy(), r["preds"].copy())
+        out[value] = (G.cpu().clone(), r["loss_adv"].copy(), r["preds"].copy())
         e.close()
-    os.environ.pop("DORPATCH_LANES", None)
-    assert torch.equal(out["1"][0], out["2"][0])
-    assert np.array_equal(out["1"][1], out["2"][1]) and np.array_equal(out["1"][2], out["2"][2])
+    a, b = (out[v] for v in settings)
+    assert torch.isfinite(a[0]).all()
+    assert torch.equal(a[0], b[0])
+    assert np.array_equal(a[1], b[1]) and np.array_equal(a[2], b[2])
 
 
 @pytest.mark.parametrize("precision", ["fp32", "bf16"])

@@ -97,12 +97,19 @@ def test_groupnorm_relu_fwd_bwd_vs_fp64(engines, precision, P, Cc, neg_gamma):
     assert ey <= tol and edx <= tol, (ey, edx)
 
 
-@pytest.mark.parametrize("B,S", [(2, 3), (1, 5)])
-def test_bf16_stem_bwd_reduce_vs_torch_fp32(engines, oracle_params, B, S):
+# (B, S, samples per launch): one launch over the whole step, and launch sequences that split images as the chunk loop does
+STEM_BWD_LAUNCHES = [(2, 3, 6), (1, 5, 5), (2, 5, 4), (3, 3, 2), (1, 7, 7)]
+
+
+@pytest.mark.parametrize("B,S,step", STEM_BWD_LAUNCHES)
+def test_bf16_stem_bwd_reduce_vs_torch_fp32(engines, oracle_params, B, S, step):
     """The K1^T the bf16 bench runs: G[b] = 2 * sum_s keep_{b,s} * conv7x7s2^T(dY_{b,s}, W) with W the standardised stem
     weights as the engine holds them (bf16), dY bf16 -- against torch fp32 conv_transpose2d on the same bf16-rounded
     operands (the factor 2 is d((x-0.5)/0.5)/dx, utils.py:77-78; keep = attack.py:206).  Both sides multiply exact
-    bf16 products and accumulate in fp32; only the summation order differs: relative L2 <= 1e-5, max abs <= 1e-4 of max."""
+    bf16 products and accumulate in fp32; only the summation order differs: relative L2 <= 1e-5, max abs <= 1e-4 of max.
+    The samples run in launches of `step` (dp_debug_k1t, samples [n0, n0 + step)) into a G that starts as NaN: the
+    launch holding an image's first sample must overwrite it, later launches add.  The split sequences also hold one
+    fully occluded sample."""
     from dorpatch_b200 import _lib, masks as PM
     e = engines("bf16")
     H, hs = 224, 112
@@ -110,19 +117,27 @@ def test_bf16_stem_bwd_reduce_vs_torch_fp32(engines, oracle_params, B, S):
     dY = (_rand((N, hs, hs, 64), 11, 1.0) * 1e-2).to(torch.bfloat16)
     idx = np.random.RandomState(7).randint(0, 2520, (B, S))
     rects = PM.gather(PM.universe(H, 2), idx)
-    G = torch.empty(B, 3, H, H, device=DEV)
-    dYd = dY.to(DEV)
     rects_c = np.ascontiguousarray(rects.reshape(N, 4, 4), np.int16)
-    _lib.check(e.lib.dp_debug_stem_bwd_reduce(e.handle, _ptr(dYd), C.c_void_p(rects_c.ctypes.data), B, S, _ptr(G), e._stream()))
+    keep = torch.from_numpy(OM.rects_to_bool(OM.universe_rects(H, 2), H))[torch.as_tensor(idx.reshape(-1))].float()
+    if step < N or N == 7:
+        rects_c[1] = 0
+        rects_c[1, 0] = (0, H, 0, H)
+        keep[1] = 0.0
+    G = torch.full((B, 3, H, H), float("nan"), device=DEV)
+    dYd = dY.to(DEV)
+    for n0 in range(0, N, step):
+        n = min(step, N - n0)
+        _lib.check(e.lib.dp_debug_k1t(e.handle, _ptr(dYd[n0:n0 + n]), C.c_void_p(rects_c.ctypes.data), B, S, n0, n, _ptr(G),
+                                      e._stream()))
     torch.cuda.synchronize()
     w = OR.standardize(oracle_params["stem.conv.weight"]).to(torch.bfloat16).float()         # [64,3,7,7]
     dX = F.conv_transpose2d(dY.float().permute(0, 3, 1, 2), w, stride=2, padding=3, output_padding=1)   # [N,3,224,224]
-    keep = torch.from_numpy(OM.rects_to_bool(OM.universe_rects(H, 2), H))[torch.as_tensor(idx.reshape(-1))].float()
     ref = 2.0 * (dX * keep).reshape(B, S, 3, H, H).sum(1)
     got = G.cpu()
+    assert torch.isfinite(got).all()
     rel = float((got - ref).norm() / ref.norm())
     mx = float((got - ref).abs().max() / ref.abs().max())
-    print("stem_bwd_reduce vs torch fp32: rel L2 %.2e, max abs / max %.2e" % (rel, mx))
+    print("stem_bwd_reduce B=%d S=%d launches of %d vs torch fp32: rel L2 %.2e, max abs / max %.2e" % (B, S, step, rel, mx))
     assert rel <= 1e-5 and mx <= 1e-4, (rel, mx)
 
 

@@ -858,6 +858,9 @@ int32_t dp_engine_create(const dp_config* cfg, dp_engine** out) {
     e->Cpd = e->bf16 ? 8 : 4;
     if (const char* s = getenv("DORPATCH_CPAD")) e->Cpd = atoi(s);
     if (e->Cpd != 4 && e->Cpd != 8) fail("DORPATCH_CPAD must be 4 or 8");
+    if (const char* gn = getenv("DORPATCH_GN"); gn && strcmp(gn, "v2") != 0)
+      fail("DORPATCH_GN=%s is no longer supported: GroupNorm always runs v2 (the two-pass kernels only on shapes v2 cannot "
+           "place); unset DORPATCH_GN or set it to v2", gn);
     const char* stem_env = getenv("DORPATCH_STEM");
     e->own_stem = e->bf16 && !(stem_env && strcmp(stem_env, "cudnn") == 0);
     e->Cp = e->own_stem ? 3 : e->Cpd;

@@ -8,8 +8,8 @@ namespace dp {
 
 constexpr int GN_GROUPS = 32;
 constexpr int GN_MAX_SPLITS = 16;
-// GroupNorm scratch (`partial`): N * GN_WS_FLOATS_PER_SAMPLE + GN_WS_FLOATS_EXTRA floats (v3: per-tile partial sums,
-// per-sample backward means, the work / done / ready counters; also covers the two-pass kernels' split partials)
+// GroupNorm scratch (`partial`): N * GN_WS_FLOATS_PER_SAMPLE + GN_WS_FLOATS_EXTRA floats: the two-pass kernels' split
+// partials, and the statistics-only kernel's per-tile partials (it runs while tiles * 64 fits GN_WS_FLOATS_PER_SAMPLE)
 constexpr int GN_WS_FLOATS_PER_SAMPLE = 8192;
 constexpr int GN_WS_FLOATS_EXTRA = 4096;
 

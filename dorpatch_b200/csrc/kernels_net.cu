@@ -8,11 +8,6 @@
 // These kernels are HBM-bound; every one is a coalesced 16-byte-vector pass.
 #include <cooperative_groups.h>
 
-#include <cstdlib>
-#include <cstring>
-#include <map>
-#include <vector>
-
 #include "common.cuh"
 #include "kernels.h"
 
@@ -96,7 +91,6 @@ void launch_unpack_nhwc(const void* in, float* dz, int N, int H, int W, int Cp, 
 // Partial group sums are combined in a fixed order (deterministic, no float atomics).
 // ------------------------------------------------------------------------------------
 constexpr int GN_THREADS = 256;
-constexpr int GN_MAXCOLS_PER_THREAD = 2;   // C/V <= 512
 
 int gn_splits(int P, int C, bool bf16) {
   const int V = bf16 ? 8 : 4;
@@ -246,7 +240,7 @@ static int apply_slabs(int P, int C, int V) {
   return s;
 }
 
-static void launch_gn_stats_v1(const void* x, float* partial, float* stats, int N, int P, int C, bool bf16, cudaStream_t st) {
+static void launch_gn_stats_2pass(const void* x, float* partial, float* stats, int N, int P, int C, bool bf16, cudaStream_t st) {
   const int splits = gn_splits(P, C, bf16);
   DISPATCH_T(bf16, (gn_stats_kernel<T><<<dim3(splits, N), GN_THREADS, 0, st>>>((const T*)x, partial, P, C, splits)));
   DISPATCH_T(bf16, (gn_finalize_kernel<T><<<N, 32, 0, st>>>(partial, stats, P, C, splits)));
@@ -361,572 +355,6 @@ void launch_gn_relu_backward_2pass(const void* dy, const void* x, const void* ad
                        (const T*)dy, (const T*)x, gamma, beta, stats, partial, P, C, splits)));
   DISPATCH_T(bf16, (gn_bwd_apply_kernel<T><<<dim3(apply_slabs(P, C, Vec<T>::N), N), GN_THREADS, 0, st>>>(
                        (const T*)dy, (const T*)x, (const T*)addend, (T*)dx, gamma, beta, stats, partial, P, C, splits)));
-}
-
-// ------------------------------------------------------------------------------------
-// Cluster-per-sample GroupNorm: ONE HBM read of the input.  A thread-block cluster of CL
-// CTAs owns one sample; each CTA pulls its contiguous pixel slab into shared memory with TMA
-// bulk copies (cp.async.bulk + mbarrier), reduces it to per-group partial sums, the cluster
-// combines the partials through distributed shared memory in rank order (deterministic), and
-// every CTA normalises its slab straight out of shared memory.
-//   forward : HBM traffic = read x + write y            (two-pass version: 2 reads + 1 write)
-//   backward: x slab stays in shared memory; dy is streamed twice (second pass hits L2, the
-//             slab was read microseconds earlier by the same SM): read x, dy (+addend), write dx.
-// ------------------------------------------------------------------------------------
-namespace gnc {
-constexpr int THREADS = 256;        // default CTA size (two CTAs per SM)
-constexpr int MAX_THREADS = 512;    // CTA size when only one CTA fits per SM (big slabs): twice the warps / loads in flight
-constexpr int MAX_GPT = 4;                       // groups per thread (V / cpg when cpg < V)
-constexpr size_t HDR = 1024;                     // mbarrier + cluster partials + stats
-__host__ __device__ constexpr size_t tp_bytes(int threads) { return (size_t)threads * MAX_GPT * 2 * sizeof(float); }
-constexpr uint32_t BULK_CHUNK = 32768;
-
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void slab_load(void* dst, const void* src, uint32_t bytes, uint64_t* bar) {
-  if (threadIdx.x == 0) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(smem_u32(bar)));
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-    for (uint32_t off = 0; off < bytes; off += BULK_CHUNK) {
-      const uint32_t nb = bytes - off < BULK_CHUNK ? bytes - off : BULK_CHUNK;
-      asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(
-                       smem_u32((const char*)dst + off)),
-                   "l"((const char*)src + off), "r"(nb), "r"(smem_u32(bar))
-                   : "memory");
-    }
-  }
-}
-__device__ __forceinline__ void slab_wait(uint64_t* bar) {
-  __syncthreads();   // the init by thread 0 is visible before anyone polls
-  uint32_t done = 0;
-  while (!done) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-        "selp.u32 %0, 1, 0, p;\n\t}"
-        : "=r"(done)
-        : "r"(smem_u32(bar)), "r"(0u)
-        : "memory");
-  }
-}
-
-// Deterministic CTA reduction of per-thread per-channel accumulators (a[V], b[V]) to per-group
-// sums; thread t owns vector column (t % cols), rows t / cols.  Result in part[g*2 + {0,1}].
-template <int V>
-__device__ __forceinline__ void cta_group_reduce(const float* a, const float* b, int C, float* tp, float* part) {
-  const int cols = C / V, cpg = C / GN_GROUPS;
-  const int gpt = cpg >= V ? 1 : V / cpg;                 // groups per thread
-  const int cpv = cpg >= V ? V : cpg;                     // channels per (thread, group)
-  // static indices only: a[] / b[] must stay in registers (dynamic indexing would spill the hot
-  // loop's accumulators to local memory)
-#pragma unroll
-  for (int j = 0; j < MAX_GPT; ++j) {
-    float sa = 0.f, sb = 0.f;
-#pragma unroll
-    for (int i = 0; i < V; ++i)
-      if (i / cpv == j) { sa += a[i]; sb += b[i]; }
-    if (j < gpt) {
-      tp[(threadIdx.x * MAX_GPT + j) * 2 + 0] = sa;
-      tp[(threadIdx.x * MAX_GPT + j) * 2 + 1] = sb;
-    }
-  }
-  __syncthreads();
-  if (threadIdx.x < GN_GROUPS) {
-    const int g = threadIdx.x, rpi = (int)blockDim.x / cols;
-    int c_lo, c_hi, j;
-    if (cpg >= V) { c_lo = g * (cpg / V); c_hi = c_lo + cpg / V; j = 0; }
-    else { c_lo = g / gpt; c_hi = c_lo + 1; j = g % gpt; }
-    float sa = 0.f, sb = 0.f;
-    for (int r = 0; r < rpi; ++r)
-      for (int c = c_lo; c < c_hi; ++c) {
-        const int t = r * cols + c;
-        sa += tp[(t * MAX_GPT + j) * 2 + 0];
-        sb += tp[(t * MAX_GPT + j) * 2 + 1];
-      }
-    part[g * 2 + 0] = sa;
-    part[g * 2 + 1] = sb;
-  }
-}
-}  // namespace gnc
-
-// Persistent variant: a cluster walks samples n = cluster_id, cluster_id + n_clusters, ... and
-// (when two slabs fit) prefetches the next sample's slab with TMA while it normalises the current one.
-namespace gnc {
-struct Pipe {
-  uint64_t* bar;      // [2] mbarriers
-  int nbuf;
-  static constexpr int CHUNK0 = 80;   // chunk barriers at byte 640 of the header; <= 7 chunks of a <= 220 KB slab
-  __device__ __forceinline__ void init() {
-    if (threadIdx.x == 0) {
-      for (int i = 0; i < 2; ++i) asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(smem_u32(bar + i)));
-      for (int i = 0; i < 8; ++i) asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(smem_u32(bar + CHUNK0 + i)));
-      asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-      asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-    }
-    __syncthreads();
-  }
-  // thread 0 only; the buffer's previous generic-proxy readers are behind a __syncthreads
-  __device__ __forceinline__ void issue(void* dst, const void* src, uint32_t bytes, int b) {
-    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar + b)), "r"(bytes) : "memory");
-    for (uint32_t off = 0; off < bytes; off += BULK_CHUNK) {
-      const uint32_t nb = bytes - off < BULK_CHUNK ? bytes - off : BULK_CHUNK;
-      asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(
-                       smem_u32((const char*)dst + off)),
-                   "l"((const char*)src + off), "r"(nb), "r"(smem_u32(bar + b))
-                   : "memory");
-    }
-  }
-  __device__ __forceinline__ void wait(int b, uint32_t parity) {
-    uint32_t done = 0;
-    while (!done) {
-      asm volatile(
-          "{\n\t.reg .pred p;\n\t"
-          "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-          "selp.u32 %0, 1, 0, p;\n\t}"
-          : "=r"(done)
-          : "r"(smem_u32(bar + b)), "r"(parity)
-          : "memory");
-    }
-  }
-  // One-shot chunked load (one cluster per sample): every 32 KB bulk copy completes on its own mbarrier
-  // (bar[CHUNK0 + k]), so the first pass over the slab starts on chunk 0 while the rest is in flight.
-  __device__ __forceinline__ void issue_chunked(void* dst, const void* src, uint32_t bytes) {   // thread 0, once, after init()
-    int k = 0;
-    for (uint32_t off = 0; off < bytes; off += BULK_CHUNK, ++k) {
-      const uint32_t nb = bytes - off < BULK_CHUNK ? bytes - off : BULK_CHUNK;
-      asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar + CHUNK0 + k)), "r"(nb) : "memory");
-      asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(
-                       smem_u32((const char*)dst + off)),
-                   "l"((const char*)src + off), "r"(nb), "r"(smem_u32(bar + CHUNK0 + k))
-                   : "memory");
-    }
-  }
-  __device__ __forceinline__ void wait_chunk(int k) { wait(CHUNK0 + k, 0u); }
-};
-}  // namespace gnc
-
-template <typename T>
-__global__ void __launch_bounds__(gnc::MAX_THREADS) gn_fwd_cluster_kernel(const T* __restrict__ x, T* __restrict__ y,
-                                                                       const float* __restrict__ gamma,
-                                                                       const float* __restrict__ beta,
-                                                                       float* __restrict__ stats, int N, int P, int C,
-                                                                       int nbuf, uint32_t slab_stride) {
-  constexpr int V = Vec<T>::N;
-  extern __shared__ __align__(128) unsigned char smem[];
-  cg::cluster_group cluster = cg::this_cluster();
-  const int CL = (int)cluster.num_blocks(), rank = (int)cluster.block_rank();
-  const int cluster_id = blockIdx.x / CL, n_clusters = gridDim.x / CL;
-  const bool chunked = nbuf == 3;   // one cluster per sample, slab loaded once through per-chunk barriers
-  gnc::Pipe pipe{reinterpret_cast<uint64_t*>(smem), nbuf};
-  float* part = reinterpret_cast<float*>(smem + 64);          // [32][2] this CTA's partials
-  float* s_mean = reinterpret_cast<float*>(smem + 64 + 256);  // [32]
-  float* s_rstd = s_mean + GN_GROUPS;                         // [32]
-  float* tp = reinterpret_cast<float*>(smem + gnc::HDR);
-  unsigned char* slabs = smem + gnc::HDR + gnc::tp_bytes((int)blockDim.x);
-
-  const int p0 = (int)(((long long)P * rank) / CL), p1 = (int)(((long long)P * (rank + 1)) / CL);
-  const int rows = p1 - p0;
-  const uint32_t slab_bytes = (uint32_t)((size_t)rows * C * sizeof(T));
-  const int cols = C / V, rpi = (int)blockDim.x / cols, cpg = C / GN_GROUPS;
-  const int tcol = threadIdx.x % cols, trow = threadIdx.x / cols;
-  pipe.init();
-
-  int it = 0;
-  for (int n = cluster_id; n < N; n += n_clusters, ++it) {
-    const int b = nbuf == 2 ? (it & 1) : 0;
-    const uint32_t parity = nbuf == 2 ? ((it >> 1) & 1) : (it & 1);
-    if (threadIdx.x == 0) {
-      if (chunked) pipe.issue_chunked(slabs, x + ((size_t)n * P + p0) * C, slab_bytes);
-      else {
-        if (it == 0 || nbuf != 2) pipe.issue(slabs + (size_t)b * slab_stride, x + ((size_t)n * P + p0) * C, slab_bytes, b);
-        if (nbuf == 2 && n + n_clusters < N)
-          pipe.issue(slabs + (size_t)(b ^ 1) * slab_stride, x + ((size_t)(n + n_clusters) * P + p0) * C, slab_bytes, b ^ 1);
-      }
-    }
-    const uint32_t toff = (uint32_t)((trow * C + tcol * V) * sizeof(T));
-    const uint32_t slab_a = gnc::smem_u32(slabs + (size_t)b * slab_stride) + toff;
-    const uint32_t srow = (uint32_t)(rpi * C * sizeof(T));
-    if (!chunked) pipe.wait(b, parity);
-
-    float a[V], bq[V];
-#pragma unroll
-    for (int i = 0; i < V; ++i) { a[i] = 0.f; bq[i] = 0.f; }
-    uint32_t sp = slab_a;
-    int have = -1;                                 // last slab chunk this thread has waited for
-    for (int r = trow; r < rows; r += rpi, sp += srow) {
-      if (chunked) {
-        const int k = (int)((sp - slab_a + toff) / gnc::BULK_CHUNK);
-        if (k != have) { pipe.wait_chunk(k); have = k; }
-      }
-      Vec<T> v; v.load_shared(sp);
-      float f[V]; v.unpack(f);
-#pragma unroll
-      for (int i = 0; i < V; ++i) { a[i] += f[i]; bq[i] = fmaf(f[i], f[i], bq[i]); }
-    }
-    gnc::cta_group_reduce<V>(a, bq, C, tp, part);
-    cluster.sync();
-    if (threadIdx.x < GN_GROUPS) {
-      float s = 0.f, q = 0.f;
-      for (int r = 0; r < CL; ++r) {
-        const float* rp = cluster.map_shared_rank(part, r);
-        s += rp[threadIdx.x * 2 + 0];
-        q += rp[threadIdx.x * 2 + 1];
-      }
-      const float cnt = (float)P * cpg;
-      const float mean = s / cnt;
-      float var = q / cnt - mean * mean;
-      var = var < 0.f ? 0.f : var;
-      const float rstd = rsqrtf(var + 1e-5f);
-      s_mean[threadIdx.x] = mean;
-      s_rstd[threadIdx.x] = rstd;
-      if (rank == 0) {
-        stats[((size_t)n * GN_GROUPS + threadIdx.x) * 2 + 0] = mean;
-        stats[((size_t)n * GN_GROUPS + threadIdx.x) * 2 + 1] = rstd;
-      }
-    }
-    __syncthreads();
-    cluster.barrier_arrive();   // our remote reads are done
-    float sa[V], sb[V];
-#pragma unroll
-    for (int i = 0; i < V; ++i) {
-      const int c = tcol * V + i, g = c / cpg;
-      sa[i] = s_rstd[g] * gamma[c];
-      sb[i] = beta[c] - s_mean[g] * sa[i];
-    }
-    T* dst = y + ((size_t)n * P + p0) * C + (size_t)trow * C + tcol * V;
-    const size_t grow = (size_t)rpi * C;
-    sp = slab_a;
-    for (int r = trow; r < rows; r += rpi, sp += srow, dst += grow) {
-      Vec<T> v; v.load_shared(sp);
-      float f[V]; v.unpack(f);
-#pragma unroll
-      for (int i = 0; i < V; ++i) f[i] = fmaxf(fmaf(sa[i], f[i], sb[i]), 0.f);
-      v.pack(f); v.store(dst);
-    }
-    __syncthreads();            // slab b, tp, s_mean free for the next iteration
-    cluster.barrier_wait();     // every peer has read our partials: `part` may be rewritten / we may exit
-  }
-}
-
-// UG: all V channels of a thread share one GroupNorm group (cpg >= V) -> per-group scalars
-template <typename T, bool UG>
-__global__ void __launch_bounds__(gnc::MAX_THREADS, 1) gn_bwd_cluster_kernel(const T* __restrict__ dy, const T* __restrict__ x,
-                                                                          const T* __restrict__ addend, T* __restrict__ dx,
-                                                                          const float* __restrict__ gamma,
-                                                                          const float* __restrict__ beta,
-                                                                          const float* __restrict__ stats, int N, int P, int C,
-                                                                          int nbuf, uint32_t slab_stride) {
-  constexpr int V = Vec<T>::N;
-#ifndef DP_GN_BWD_U
-#define DP_GN_BWD_U 4
-#endif
-  constexpr int U = DP_GN_BWD_U;   // independent global loads in flight per thread (plus the TMA slab)
-  constexpr int GV = UG ? 1 : V;
-  extern __shared__ __align__(128) unsigned char smem[];
-  cg::cluster_group cluster = cg::this_cluster();
-  const int CL = (int)cluster.num_blocks(), rank = (int)cluster.block_rank();
-  const int cluster_id = blockIdx.x / CL, n_clusters = gridDim.x / CL;
-  const bool chunked = nbuf == 3;   // one cluster per sample, x slab loaded once through per-chunk barriers
-  gnc::Pipe pipe{reinterpret_cast<uint64_t*>(smem), nbuf};
-  float* part = reinterpret_cast<float*>(smem + 64);
-  float* s_1 = reinterpret_cast<float*>(smem + 64 + 256);
-  float* s_2 = s_1 + GN_GROUPS;
-  float* tp = reinterpret_cast<float*>(smem + gnc::HDR);
-  unsigned char* slabs = smem + gnc::HDR + gnc::tp_bytes((int)blockDim.x);
-
-  const int p0 = (int)(((long long)P * rank) / CL), p1 = (int)(((long long)P * (rank + 1)) / CL);
-  const int rows = p1 - p0;
-  const uint32_t slab_bytes = (uint32_t)((size_t)rows * C * sizeof(T));
-  const int cols = C / V, rpi = (int)blockDim.x / cols, cpg = C / GN_GROUPS;
-  const int tcol = threadIdx.x % cols, trow = threadIdx.x / cols;
-  float ga[V];
-#pragma unroll
-  for (int i = 0; i < V; ++i) ga[i] = gamma[tcol * V + i];
-  pipe.init();
-
-  int it = 0;
-  for (int n = cluster_id; n < N; n += n_clusters, ++it) {
-    const int b = nbuf == 2 ? (it & 1) : 0;
-    const uint32_t parity = nbuf == 2 ? ((it >> 1) & 1) : (it & 1);
-    const size_t base = ((size_t)n * P + p0) * C;
-    if (threadIdx.x == 0) {
-      if (chunked) pipe.issue_chunked(slabs, x + base, slab_bytes);
-      else {
-        if (it == 0 || nbuf != 2) pipe.issue(slabs + (size_t)b * slab_stride, x + base, slab_bytes, b);
-        if (nbuf == 2 && n + n_clusters < N)
-          pipe.issue(slabs + (size_t)(b ^ 1) * slab_stride, x + ((size_t)(n + n_clusters) * P + p0) * C, slab_bytes, b ^ 1);
-      }
-    }
-    const uint32_t slab_a = gnc::smem_u32(slabs + (size_t)b * slab_stride) + (uint32_t)(tcol * V * sizeof(T));
-    const uint32_t crow = (uint32_t)(C * sizeof(T));
-    float sa[V], sb[V], mu[GV], rs[GV];
-#pragma unroll
-    for (int i = 0; i < GV; ++i) {
-      const int g = (tcol * V + i) / cpg;
-      mu[i] = stats[((size_t)n * GN_GROUPS + g) * 2 + 0];
-      rs[i] = stats[((size_t)n * GN_GROUPS + g) * 2 + 1];
-    }
-#pragma unroll
-    for (int i = 0; i < V; ++i) {
-      sa[i] = rs[UG ? 0 : i] * ga[i];
-      sb[i] = beta[tcol * V + i] - mu[UG ? 0 : i] * sa[i];
-    }
-    if (!chunked) pipe.wait(b, parity);
-    float a[V], bq[V];
-#pragma unroll
-    for (int i = 0; i < V; ++i) { a[i] = 0.f; bq[i] = 0.f; }
-    int have = -1;                                 // last slab chunk this thread has waited for
-    for (int r0 = trow; r0 < rows; r0 += rpi * U) {
-      Vec<T> vd[U];
-#pragma unroll
-      for (int u = 0; u < U; ++u) {
-        const int r = r0 + u * rpi;
-        if (r < rows) vd[u].load(dy + base + (size_t)r * C + tcol * V);
-      }
-#pragma unroll
-      for (int u = 0; u < U; ++u) {
-        const int r = r0 + u * rpi;
-        if (r < rows) {
-          if (chunked) {
-            const int k = (int)(((uint32_t)r * crow + (uint32_t)(tcol * V * sizeof(T))) / gnc::BULK_CHUNK);
-            if (k != have) { pipe.wait_chunk(k); have = k; }
-          }
-          Vec<T> vx; vx.load_shared(slab_a + (uint32_t)r * crow);
-          float fx[V], fd[V]; vx.unpack(fx); vd[u].unpack(fd);
-#pragma unroll
-          for (int i = 0; i < V; ++i) {
-            const float pre = fmaf(sa[i], fx[i], sb[i]);
-            const float dg = pre > 0.f ? fd[i] * ga[i] : 0.f;
-            const float xh = (fx[i] - mu[UG ? 0 : i]) * rs[UG ? 0 : i];
-            a[i] += dg; bq[i] = fmaf(dg, xh, bq[i]);
-          }
-        }
-      }
-    }
-    gnc::cta_group_reduce<V>(a, bq, C, tp, part);
-    cluster.sync();
-    if (threadIdx.x < GN_GROUPS) {
-      float s = 0.f, q = 0.f;
-      for (int r = 0; r < CL; ++r) {
-        const float* rp = cluster.map_shared_rank(part, r);
-        s += rp[threadIdx.x * 2 + 0];
-        q += rp[threadIdx.x * 2 + 1];
-      }
-      const float inv_m = 1.0f / ((float)P * cpg);
-      s_1[threadIdx.x] = s * inv_m;
-      s_2[threadIdx.x] = q * inv_m;
-    }
-    __syncthreads();
-    cluster.barrier_arrive();
-    float m1[GV], m2[GV];
-#pragma unroll
-    for (int i = 0; i < GV; ++i) { const int g = (tcol * V + i) / cpg; m1[i] = s_1[g]; m2[i] = s_2[g]; }
-    for (int r0 = trow; r0 < rows; r0 += rpi * U) {
-      Vec<T> vd[U], va[U];
-#pragma unroll
-      for (int u = 0; u < U; ++u) {
-        const int r = r0 + u * rpi;
-        if (r < rows) {
-          const size_t off = base + (size_t)r * C + tcol * V;
-          vd[u].load(dy + off);
-          if (addend != nullptr) va[u].load(addend + off);
-        }
-      }
-#pragma unroll
-      for (int u = 0; u < U; ++u) {
-        const int r = r0 + u * rpi;
-        if (r < rows) {
-          const size_t off = base + (size_t)r * C + tcol * V;
-          Vec<T> vx; vx.load_shared(slab_a + (uint32_t)r * crow);
-          float fx[V], fd[V], fo[V]; vx.unpack(fx); vd[u].unpack(fd);
-          if (addend != nullptr) va[u].unpack(fo);
-          else {
-#pragma unroll
-            for (int i = 0; i < V; ++i) fo[i] = 0.f;
-          }
-#pragma unroll
-          for (int i = 0; i < V; ++i) {
-            const float pre = fmaf(sa[i], fx[i], sb[i]);
-            const float dg = pre > 0.f ? fd[i] * ga[i] : 0.f;
-            const float xh = (fx[i] - mu[UG ? 0 : i]) * rs[UG ? 0 : i];
-            fo[i] += rs[UG ? 0 : i] * (dg - m1[UG ? 0 : i] - xh * m2[UG ? 0 : i]);
-          }
-          Vec<T> vo; vo.pack(fo); vo.store(dx + off);
-        }
-      }
-    }
-    __syncthreads();
-    cluster.barrier_wait();
-  }
-}
-
-// Backward variant with BOTH x and dy slabs resident in shared memory (two TMA loads issued up front,
-// no global-load latency chains in either pass).  One cluster per sample; used when two slabs fit the
-// per-CTA budget.
-template <typename T, bool UG>
-__global__ void __launch_bounds__(gnc::MAX_THREADS, 1) gn_bwd_cluster_smem_kernel(const T* __restrict__ dy, const T* __restrict__ x,
-                                                                               const T* __restrict__ addend, T* __restrict__ dx,
-                                                                               const float* __restrict__ gamma,
-                                                                               const float* __restrict__ beta,
-                                                                               const float* __restrict__ stats, int P, int C,
-                                                                               uint32_t slab_stride) {
-  constexpr int V = Vec<T>::N;
-  constexpr int GV = UG ? 1 : V;
-  extern __shared__ __align__(128) unsigned char smem[];
-  cg::cluster_group cluster = cg::this_cluster();
-  const int CL = (int)cluster.num_blocks(), rank = (int)cluster.block_rank();
-  const int n = blockIdx.x / CL;
-  gnc::Pipe pipe{reinterpret_cast<uint64_t*>(smem), 2};
-  float* part = reinterpret_cast<float*>(smem + 64);
-  float* s_1 = reinterpret_cast<float*>(smem + 64 + 256);
-  float* s_2 = s_1 + GN_GROUPS;
-  float* tp = reinterpret_cast<float*>(smem + gnc::HDR);
-  unsigned char* slabs = smem + gnc::HDR + gnc::tp_bytes((int)blockDim.x);
-
-  const int p0 = (int)(((long long)P * rank) / CL), p1 = (int)(((long long)P * (rank + 1)) / CL);
-  const int rows = p1 - p0;
-  const uint32_t slab_bytes = (uint32_t)((size_t)rows * C * sizeof(T));
-  const size_t base = ((size_t)n * P + p0) * C;
-  const int cols = C / V, rpi = (int)blockDim.x / cols, cpg = C / GN_GROUPS;
-  const int tcol = threadIdx.x % cols, trow = threadIdx.x / cols;
-  pipe.init();
-  if (threadIdx.x == 0) {
-    pipe.issue(slabs, x + base, slab_bytes, 0);
-    pipe.issue(slabs + slab_stride, dy + base, slab_bytes, 1);
-  }
-  float ga[V], sa[V], sb[V], mu[GV], rs[GV];
-#pragma unroll
-  for (int i = 0; i < GV; ++i) {
-    const int g = (tcol * V + i) / cpg;
-    mu[i] = stats[((size_t)n * GN_GROUPS + g) * 2 + 0];
-    rs[i] = stats[((size_t)n * GN_GROUPS + g) * 2 + 1];
-  }
-#pragma unroll
-  for (int i = 0; i < V; ++i) {
-    ga[i] = gamma[tcol * V + i];
-    sa[i] = rs[UG ? 0 : i] * ga[i];
-    sb[i] = beta[tcol * V + i] - mu[UG ? 0 : i] * sa[i];
-  }
-  const uint32_t xa = gnc::smem_u32(slabs) + (uint32_t)((trow * C + tcol * V) * sizeof(T));
-  const uint32_t da = xa + slab_stride;
-  const uint32_t srow = (uint32_t)(rpi * C * sizeof(T));
-  pipe.wait(0, 0);
-  pipe.wait(1, 0);
-  float a[V], bq[V];
-#pragma unroll
-  for (int i = 0; i < V; ++i) { a[i] = 0.f; bq[i] = 0.f; }
-  uint32_t off = 0;
-  for (int r = trow; r < rows; r += rpi, off += srow) {
-    Vec<T> vx, vd; vx.load_shared(xa + off); vd.load_shared(da + off);
-    float fx[V], fd[V]; vx.unpack(fx); vd.unpack(fd);
-#pragma unroll
-    for (int i = 0; i < V; ++i) {
-      const float pre = fmaf(sa[i], fx[i], sb[i]);
-      const float dg = pre > 0.f ? fd[i] * ga[i] : 0.f;
-      const float xh = (fx[i] - mu[UG ? 0 : i]) * rs[UG ? 0 : i];
-      a[i] += dg; bq[i] = fmaf(dg, xh, bq[i]);
-    }
-  }
-  gnc::cta_group_reduce<V>(a, bq, C, tp, part);
-  cluster.sync();
-  if (threadIdx.x < GN_GROUPS) {
-    float s = 0.f, q = 0.f;
-    for (int r = 0; r < CL; ++r) {
-      const float* rp = cluster.map_shared_rank(part, r);
-      s += rp[threadIdx.x * 2 + 0];
-      q += rp[threadIdx.x * 2 + 1];
-    }
-    const float inv_m = 1.0f / ((float)P * cpg);
-    s_1[threadIdx.x] = s * inv_m;
-    s_2[threadIdx.x] = q * inv_m;
-  }
-  __syncthreads();
-  cluster.barrier_arrive();
-  float m1[GV], m2[GV];
-#pragma unroll
-  for (int i = 0; i < GV; ++i) { const int g = (tcol * V + i) / cpg; m1[i] = s_1[g]; m2[i] = s_2[g]; }
-  const size_t grow = (size_t)rpi * C;
-  size_t goff = base + (size_t)trow * C + tcol * V;
-  off = 0;
-  for (int r = trow; r < rows; r += rpi, off += srow, goff += grow) {
-    Vec<T> vx, vd; vx.load_shared(xa + off); vd.load_shared(da + off);
-    float fx[V], fd[V], fo[V]; vx.unpack(fx); vd.unpack(fd);
-    if (addend != nullptr) { Vec<T> va; va.load(addend + goff); va.unpack(fo); }
-    else {
-#pragma unroll
-      for (int i = 0; i < V; ++i) fo[i] = 0.f;
-    }
-#pragma unroll
-    for (int i = 0; i < V; ++i) {
-      const float pre = fmaf(sa[i], fx[i], sb[i]);
-      const float dg = pre > 0.f ? fd[i] * ga[i] : 0.f;
-      const float xh = (fx[i] - mu[UG ? 0 : i]) * rs[UG ? 0 : i];
-      fo[i] += rs[UG ? 0 : i] * (dg - m1[UG ? 0 : i] - xh * m2[UG ? 0 : i]);
-    }
-    Vec<T> vo; vo.pack(fo); vo.store(dx + goff);
-  }
-  cluster.barrier_wait();
-}
-
-struct GnPlan { int cl; int nbuf; size_t smem; uint32_t slab_stride; int ctas_per_sm; bool persistent; int threads; };
-// Tunables (environment, read once): DORPATCH_GN=twopass disables the cluster kernels;
-// DORPATCH_GN_PERSIST=1 -> persistent clusters with double-buffered slab prefetch (measured slower on
-// B200 than one cluster per sample: fewer resident CTAs); DORPATCH_GN_SOFT=<KB> per-CTA smem budget
-// used to pick the cluster size.
-static bool gn_plan(int P, int C, size_t es, GnPlan* out) {
-  static int mode = -1, persist = 0, big_threads = gnc::MAX_THREADS, cl16 = 0;
-  static size_t soft = 111 * 1024;
-  if (mode < 0) {
-    const char* e = getenv("DORPATCH_GN"); mode = (e && strcmp(e, "twopass") == 0) ? 0 : 1;
-    if (const char* p = getenv("DORPATCH_GN_PERSIST")) persist = atoi(p);
-    if (const char* q = getenv("DORPATCH_GN_SOFT")) soft = (size_t)atoi(q) * 1024;
-    if (const char* t = getenv("DORPATCH_GN_BIGTHREADS")) big_threads = atoi(t);
-    if (const char* c = getenv("DORPATCH_GN_CL16")) cl16 = atoi(c);   // non-portable cluster size 16 for the biggest slabs
-  }
-  if (!mode) return false;
-  if (C / (int)(16 / es) > gnc::THREADS) return false;
-  const size_t fixed = gnc::HDR + gnc::tp_bytes(gnc::THREADS), fixed_big = gnc::HDR + gnc::tp_bytes(big_threads), hard = 220 * 1024;
-  for (int cl = 1; cl <= 8; cl *= 2) {
-    if (cl > P) break;
-    const size_t slab = (((size_t)((P + cl - 1) / cl)) * C * es + 127) / 128 * 128;
-    if (persist) {
-      if (fixed + 2 * slab <= soft) { *out = GnPlan{cl, 2, fixed + 2 * slab, (uint32_t)slab, (int)(hard / (fixed + 2 * slab)), true, gnc::THREADS}; return true; }
-      if (cl == 8) {
-        if (fixed + 2 * slab <= hard) { *out = GnPlan{cl, 2, fixed + 2 * slab, (uint32_t)slab, 1, true, gnc::THREADS}; return true; }
-        if (fixed + slab <= hard) { *out = GnPlan{cl, 1, fixed + slab, (uint32_t)slab, 1, true, gnc::THREADS}; return true; }
-      }
-    } else if (fixed + slab <= soft) {
-      *out = GnPlan{cl, 1, fixed + slab, (uint32_t)slab, 1, false, gnc::THREADS};
-      return true;
-    } else if (cl == 8 && cl16 && P >= 16 && fixed + (slab + 1) / 2 + 128 <= soft) {
-      const size_t slab16 = (((size_t)((P + 15) / 16)) * C * es + 127) / 128 * 128;
-      *out = GnPlan{16, 1, fixed + slab16, (uint32_t)slab16, 1, false, gnc::THREADS};
-      return true;
-    } else if (cl == 8 && fixed_big + slab <= hard) {
-      // a slab that leaves room for only one CTA per SM gets a 512-thread CTA
-      *out = GnPlan{cl, 1, fixed_big + slab, (uint32_t)slab, 1, false, big_threads};
-      return true;
-    }
-  }
-  return false;
-}
-// DORPATCH_GN_CHUNKED (default 1; 0 = one barrier for the whole slab): one-cluster-per-sample launches load the slab through per-32KB mbarriers
-// (kernel argument nbuf = 3) so the statistics pass overlaps the tail of the TMA load.
-static int gn_nbuf(const GnPlan& pl) {
-  static int chunked = -1;
-  if (chunked < 0) { const char* e = getenv("DORPATCH_GN_CHUNKED"); chunked = e ? atoi(e) : 1; }
-  return (!pl.persistent && chunked) ? 3 : pl.nbuf;
-}
-static int g_num_sms = 0;
-static int gn_grid(const GnPlan& pl, int N) {
-  if (!pl.persistent) return pl.cl * N;                       // one cluster per sample
-  if (g_num_sms == 0) { int dev = 0; cudaGetDevice(&dev); cudaDeviceGetAttribute(&g_num_sms, cudaDevAttrMultiProcessorCount, dev); }
-  int n_clusters = (g_num_sms * pl.ctas_per_sm) / pl.cl;
-  if (n_clusters < 1) n_clusters = 1;
-  if (n_clusters > N) n_clusters = N;
-  return n_clusters * pl.cl;
 }
 
 template <typename K, typename... Args>
@@ -1161,12 +589,16 @@ void launch_subsample2_adjoint_add(const void* dy, void* dx, int N, int H, int W
   });
 }
 
-
 // ====================================================================================
-// GroupNorm v2 (round 2): the same cluster-per-sample scheme, rebuilt for instruction count.
-// ncu of v1 (profiles/r02_gn_v1_ncu.txt): DRAM traffic = algorithmic, but 330 warp-instructions per
-// 16-byte (x, dy) vector pair at IPC 1.5 -- 64-bit address arithmetic, per-row bound / chunk checks and
-// per-element unpack + gate dominate; the kernels are issue-bound, not HBM-bound.  v2:
+// GroupNorm v2, cluster per sample: ONE HBM read of the input.  A thread-block cluster of CL CTAs owns one sample;
+// each CTA pulls its contiguous pixel slab into shared memory with TMA bulk copies (cp.async.bulk + mbarrier), reduces
+// it to per-group partial sums, the cluster combines the partials through distributed shared memory in rank order
+// (deterministic), and every CTA normalises its slab straight out of shared memory.  Shapes the plan below cannot
+// place (slab too large, C/V > 256) run on the two-pass kernels above.
+// Written against the round-1 cluster kernels (ncu: profiles/r02_gn_fwd_v1_ncu.txt, r02_gn_bwd_v1_ncu.txt): DRAM
+// traffic = algorithmic, but 330 warp-instructions per 16-byte (x, dy) vector pair at IPC 1.5 -- 64-bit address
+// arithmetic, per-row bound / chunk checks and per-element unpack + gate dominate; those kernels were issue-bound, not
+// HBM-bound.  v2:
 //   * a CTA's slab is a LINEAR array of 16-byte vectors; thread t owns vectors t, t + T, t + 2T, ... (its channel
 //     column is fixed because T % (C/V) == 0), so the loops carry one 32-bit offset and no row / column arithmetic;
 //   * the TMA load completes on one mbarrier per 32 KB chunk and the loops walk whole chunks (IPC iterations,
@@ -1184,6 +616,9 @@ __device__ unsigned long long* g_trace = nullptr;   // optional phase trace (too
 constexpr uint32_t CHUNK = 32768;
 constexpr int MAX_CHUNKS = 7;                      // <= 224 KB per slab
 constexpr int OFF_BAR_X = 0, OFF_BAR_D = 64, OFF_PART = 128, OFF_SA = 384, OFF_SB = 512, OFF_FLAG = 640;
+constexpr size_t HDR = 1024;                       // the OFF_* fields above; the reduction scratch follows, then the slab(s)
+constexpr int MAX_GPT = 4;                         // groups per thread (V / cpg when cpg < V)
+__host__ __device__ constexpr size_t tp_bytes(int threads) { return (size_t)threads * MAX_GPT * 2 * sizeof(float); }
 
 __device__ __forceinline__ uint32_t s32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
 __device__ __forceinline__ void bar_init(uint32_t bar) { asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(bar)); }
@@ -1276,8 +711,9 @@ template <> struct Acc<__nv_bfloat16> {
 
 // Deterministic CTA reduction of per-thread per-channel accumulators (a[V], b[V]) to the 32 per-group sums, for the
 // linear thread -> column mapping (column = threadIdx.x % cols): fixed xor-shuffle tree inside each warp, one
-// shared-memory exchange, fixed-order sum over the warps.  ~300 cycles; the shared-memory loop of gnc::cta_group_reduce
-// it replaces took 3-9k cycles per slab (phase trace, profiles/r02_gn_v2_trace.txt).  red: >= (blockDim/32) * 64 floats.
+// shared-memory exchange, fixed-order sum over the warps.  ~300 cycles; the shared-memory reduction loop of the round-1
+// kernels (profiles/r02_gn_*_v1_ncu.txt) took 3-9k cycles per slab (tools/gnbench.cu phase trace).
+// red: >= (blockDim/32) * 64 floats.
 template <int V>
 __device__ __forceinline__ void group_reduce(const float* a, const float* b, int C, float* red, float* part) {
   const int cols = C / V, cpg = C / GN_GROUPS;
@@ -1285,9 +721,9 @@ __device__ __forceinline__ void group_reduce(const float* a, const float* b, int
   if (cpg <= V) {
     // each thread holds gpt = V / cpg whole groups; threads of one column sit `cols` lanes apart (cols <= 32)
     const int gpt = V / cpg;
-    float sa[gnc::MAX_GPT], sb[gnc::MAX_GPT];
+    float sa[MAX_GPT], sb[MAX_GPT];
 #pragma unroll
-    for (int j = 0; j < gnc::MAX_GPT; ++j) {
+    for (int j = 0; j < MAX_GPT; ++j) {
       sa[j] = 0.f; sb[j] = 0.f;
 #pragma unroll
       for (int i = 0; i < V; ++i)
@@ -1295,7 +731,7 @@ __device__ __forceinline__ void group_reduce(const float* a, const float* b, int
     }
     for (int o = cols; o < 32; o <<= 1) {
 #pragma unroll
-      for (int j = 0; j < gnc::MAX_GPT; ++j) {
+      for (int j = 0; j < MAX_GPT; ++j) {
         sa[j] += __shfl_xor_sync(0xffffffffu, sa[j], o);
         sb[j] += __shfl_xor_sync(0xffffffffu, sb[j], o);
       }
@@ -1303,7 +739,7 @@ __device__ __forceinline__ void group_reduce(const float* a, const float* b, int
     __syncthreads();                                  // `red` may still be read by the previous use
     if (lane < cols) {
 #pragma unroll
-      for (int j = 0; j < gnc::MAX_GPT; ++j)
+      for (int j = 0; j < MAX_GPT; ++j)
         if (j < gpt) { red[warp * 64 + (lane * gpt + j) * 2 + 0] = sa[j]; red[warp * 64 + (lane * gpt + j) * 2 + 1] = sb[j]; }
     }
     __syncthreads();
@@ -1392,8 +828,8 @@ __global__ void __launch_bounds__(TH, TH == 256 ? 2 : 1) fwd_kernel(const T* __r
   float* part = reinterpret_cast<float*>(smem + OFF_PART);
   float* s_mean = reinterpret_cast<float*>(smem + OFF_SA);
   float* s_rstd = reinterpret_cast<float*>(smem + OFF_SB);
-  float* tp = reinterpret_cast<float*>(smem + gnc::HDR);
-  const uint32_t slab = sb0 + (uint32_t)(gnc::HDR + gnc::tp_bytes(TH));
+  float* tp = reinterpret_cast<float*>(smem + HDR);
+  const uint32_t slab = sb0 + (uint32_t)(HDR + tp_bytes(TH));
 
   const int p0 = (int)(((long long)P * rank) / CL), p1 = (int)(((long long)P * (rank + 1)) / CL);
   const uint32_t slab_bytes = (uint32_t)((size_t)(p1 - p0) * C * sizeof(T));
@@ -1518,8 +954,8 @@ __global__ void __launch_bounds__(TH, TH == 256 ? 2 : 1) bwd_kernel(const T* __r
   float* part = reinterpret_cast<float*>(smem + OFF_PART);
   float* s_1 = reinterpret_cast<float*>(smem + OFF_SA);
   float* s_2 = reinterpret_cast<float*>(smem + OFF_SB);
-  float* tp = reinterpret_cast<float*>(smem + gnc::HDR);
-  const uint32_t xs = sb0 + (uint32_t)(gnc::HDR + gnc::tp_bytes(TH));
+  float* tp = reinterpret_cast<float*>(smem + HDR);
+  const uint32_t xs = sb0 + (uint32_t)(HDR + tp_bytes(TH));
   const uint32_t ds = xs + slab_stride;
 
   const int p0 = (int)(((long long)P * rank) / CL), p1 = (int)(((long long)P * (rank + 1)) / CL);
@@ -1696,420 +1132,54 @@ __global__ void __launch_bounds__(TH, TH == 256 ? 2 : 1) bwd_kernel(const T* __r
 struct Plan { int cl, threads; bool dys; size_t smem; uint32_t stride; };
 }  // namespace gn2
 
-
-// ====================================================================================
-// GroupNorm v3: streaming two-phase kernel, second read from L2 (no clusters, no slab in shared memory).
-// Phase traces of v2 (tools/gnbench.cu, profiles/r02_gn_v2_trace.txt) show where a cluster-per-sample kernel loses:
-// one 200 KB slab per SM serialises load -> statistics -> cluster barrier (2-3k cycles of skew) -> DSMEM finalize ->
-// apply, clusters of 8 strand 20 of 148 SMs (GPCs hold 16-20 SMs), and 16 warps per SM cannot hide any of it --
-// while a plain two-pass pair of kernels streams at 90 % of peak but moves 3 units instead of 2.  v3 keeps the
-// streaming structure AND the 2-unit traffic: a persistent grid pulls work items (sample, 32-64 KB tile, phase) from a
-// global counter, ordered so that a group of G samples (G x sample bytes ~ 24 MB, far inside the 126 MB L2) has all its
-// phase-1 items (read x, per-tile group sums -> global partials, count) ahead of its phase-2 items (wait for the
-// sample's statistics flag, re-read the tile -- an L2 hit --, normalise, write).  The last tile of a sample reduces the
-// partials in tile order (deterministic) and publishes mean / rstd.  Phase-1 items never wait, items are handed out in
-// order, so a phase-2 item only ever waits for items already running: no co-residency assumption, no deadlock.
-// HBM traffic: forward 1 read + 1 write, backward reads of x, dy (+ addend) + 1 write.
-// ====================================================================================
-namespace gn3 {
-using gn2::Acc;
-constexpr int TH = 256;
-constexpr int CTL_WORDS = 32;   // [0] work counter; done[n] at CTL_WORDS + n; ready[n] at CTL_WORDS + N + n
-
-__device__ __forceinline__ unsigned ld_acquire(const unsigned* p) {
-  unsigned v;
-  asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
-  return v;
-}
-struct Item { int n, t, phase; };
-__device__ __forceinline__ bool next_item(unsigned* ctl, unsigned* s_item, int N, int G, int tiles, Item& it) {
-  __syncthreads();                                   // everyone is done with the previous item (and with *s_item)
-  if (threadIdx.x == 0) *s_item = atomicAdd(ctl, 1u);
-  __syncthreads();
-  const unsigned i = *s_item, per = 2u * (unsigned)G * (unsigned)tiles;
-  const unsigned g = i / per;
-  const int n0 = (int)g * G;
-  if (n0 >= N) return false;
-  const int ng = min(G, N - n0);
-  unsigned r = i - g * per;
-  if (r >= 2u * (unsigned)ng * (unsigned)tiles) return false;      // past the (partial) last group
-  it.phase = r >= (unsigned)ng * (unsigned)tiles ? 1 : 0;
-  r -= (unsigned)it.phase * (unsigned)ng * (unsigned)tiles;
-  it.n = n0 + (int)(r / (unsigned)tiles);
-  it.t = (int)(r % (unsigned)tiles);
-  return true;
-}
-// per-tile group sums -> global partial; the sample's last tile reduces all partials in tile order and publishes
-// out2[n][g] = finish(sum_a, sum_b); then raises ready[n].
-template <int V, typename F>
-__device__ __forceinline__ void publish(const float* a, const float* b, int C, float* tp, float* part, float* partial,
-                                        unsigned* ctl, int N, int n, int t, int tiles, unsigned* s_flag, float* out2, F&& finish) {
-  gnc::cta_group_reduce<V>(a, b, C, tp, part);
-  float* pt = partial + ((size_t)n * tiles + t) * (GN_GROUPS * 2);
-  if (threadIdx.x < GN_GROUPS) {
-    pt[threadIdx.x * 2 + 0] = part[threadIdx.x * 2 + 0];
-    pt[threadIdx.x * 2 + 1] = part[threadIdx.x * 2 + 1];
-    __threadfence();
-  }
-  __syncthreads();
-  if (threadIdx.x == 0) *s_flag = (atomicAdd(ctl + CTL_WORDS + n, 1u) == (unsigned)(tiles - 1)) ? 1u : 0u;
-  __syncthreads();
-  if (*s_flag) {
-    if (threadIdx.x < GN_GROUPS) {
-      __threadfence();
-      float sa = 0.f, sb = 0.f;
-      const float* pn = partial + (size_t)n * tiles * (GN_GROUPS * 2);
-      for (int k = 0; k < tiles; ++k) {
-        sa += __ldcg(pn + (size_t)k * (GN_GROUPS * 2) + threadIdx.x * 2 + 0);
-        sb += __ldcg(pn + (size_t)k * (GN_GROUPS * 2) + threadIdx.x * 2 + 1);
-      }
-      float o0, o1;
-      finish(sa, sb, o0, o1);
-      out2[((size_t)n * GN_GROUPS + threadIdx.x) * 2 + 0] = o0;
-      out2[((size_t)n * GN_GROUPS + threadIdx.x) * 2 + 1] = o1;
-      __threadfence();
-    }
-    __syncthreads();
-    if (threadIdx.x == 0) atomicExch(ctl + CTL_WORDS + N + n, 1u);
-  }
-}
-__device__ __forceinline__ void wait_ready(unsigned* ctl, int N, int n) {
-  if (threadIdx.x == 0) while (ld_acquire(ctl + CTL_WORDS + N + n) == 0u) __nanosleep(100);
-  __syncthreads();
-}
-
-template <typename T, int ITER>
-__global__ void __launch_bounds__(TH, 4) fwd_kernel(const T* __restrict__ x, T* __restrict__ y, const float* __restrict__ gamma,
-                                                 const float* __restrict__ beta, float* __restrict__ stats, float* __restrict__ partial,
-                                                 unsigned* __restrict__ ctl, int N, int P, int C, int G, int tiles) {
-  using A = Acc<T>;
-  constexpr int V = A::V;
-  constexpr int UB = 8;                                  // vectors in flight per thread
-  __shared__ float tp[TH * gnc::MAX_GPT * 2];
-  __shared__ float part[GN_GROUPS * 2];
-  __shared__ unsigned s_item, s_flag;
-  const int cols = C / V, cpg = C / GN_GROUPS, tcol = threadIdx.x % cols;
-  const uint32_t sample_vecs = (uint32_t)P * cols;
-  const float cnt = (float)P * cpg;
-  Item it;
-  while (next_item(ctl, &s_item, N, G, tiles, it)) {
-    const char* xs = reinterpret_cast<const char*>(x) + (size_t)it.n * sample_vecs * 16;
-    const uint32_t v0 = (uint32_t)it.t * TH * ITER + threadIdx.x;
-    if (it.phase == 0) {
-      float a[V], bq[V];
-#pragma unroll
-      for (int i = 0; i < V; ++i) { a[i] = 0.f; bq[i] = 0.f; }
-#pragma unroll
-      for (int j0 = 0; j0 < ITER; j0 += UB) {
-        uint4 v[UB];
-#pragma unroll
-        for (int j = 0; j < UB; ++j) {
-          const uint32_t vi = v0 + (j0 + j) * TH;
-          v[j] = vi < sample_vecs ? gn2::ldg128(xs + (size_t)vi * 16) : make_uint4(0u, 0u, 0u, 0u);
-        }
-#pragma unroll
-        for (int j = 0; j < UB; ++j) {
-          float f[V]; A::unpack(v[j], f);
-#pragma unroll
-          for (int i = 0; i < V; ++i) { a[i] += f[i]; bq[i] = fmaf(f[i], f[i], bq[i]); }
-        }
-      }
-      publish<V>(a, bq, C, tp, part, partial, ctl, N, it.n, it.t, tiles, &s_flag, stats, [&](float s, float q, float& o0, float& o1) {
-        const float mean = s / cnt;
-        float var = q / cnt - mean * mean;
-        var = var < 0.f ? 0.f : var;
-        o0 = mean; o1 = rsqrtf(var + 1e-5f);
-      });
-    } else {
-      wait_ready(ctl, N, it.n);
-      float sa[V], sb[V];
-#pragma unroll
-      for (int i = 0; i < V; ++i) {
-        const int c = tcol * V + i, g = c / cpg;
-        const float mean = __ldcg(stats + ((size_t)it.n * GN_GROUPS + g) * 2), rstd = __ldcg(stats + ((size_t)it.n * GN_GROUPS + g) * 2 + 1);
-        sa[i] = rstd * gamma[c];
-        sb[i] = beta[c] - mean * sa[i];
-      }
-      char* ys = reinterpret_cast<char*>(y) + (size_t)it.n * sample_vecs * 16;
-#pragma unroll
-      for (int j0 = 0; j0 < ITER; j0 += UB) {
-        uint4 v[UB];
-#pragma unroll
-        for (int j = 0; j < UB; ++j) {
-          const uint32_t vi = v0 + (j0 + j) * TH;
-          v[j] = vi < sample_vecs ? gn2::ldg128(xs + (size_t)vi * 16) : make_uint4(0u, 0u, 0u, 0u);
-        }
-#pragma unroll
-        for (int j = 0; j < UB; ++j) {
-          const uint32_t vi = v0 + (j0 + j) * TH;
-          if (vi < sample_vecs) *reinterpret_cast<uint4*>(ys + (size_t)vi * 16) = A::apply_relu(v[j], sa, sb);
-        }
-      }
-    }
-  }
-}
-
-// backward: phase 1 sums dg and dg*xhat per group (dg = dy * gate * gamma), phase 2 writes dx = k1*dym + k2*x + k3 (+ addend)
-template <typename T, int ITER, bool NEG>
-__global__ void __launch_bounds__(TH, 3) bwd_kernel(const T* __restrict__ dy, const T* __restrict__ x, const T* __restrict__ addend,
-                                                 T* __restrict__ dx, const float* __restrict__ gamma, const float* __restrict__ beta,
-                                                 const float* __restrict__ stats, float* __restrict__ partial, float* __restrict__ m12,
-                                                 unsigned* __restrict__ ctl, int N, int P, int C, int G, int tiles) {
-  using A = Acc<T>;
-  constexpr int V = A::V;
-  constexpr bool PACKED = sizeof(T) == 2 && !NEG;
-  constexpr int UB = 4;
-  __shared__ float tp[TH * gnc::MAX_GPT * 2];
-  __shared__ float part[GN_GROUPS * 2];
-  __shared__ unsigned s_item, s_flag;
-  const int cols = C / V, cpg = C / GN_GROUPS, tcol = threadIdx.x % cols;
-  const uint32_t sample_vecs = (uint32_t)P * cols;
-  const float inv_m = 1.0f / ((float)P * cpg);
-  Item it;
-  while (next_item(ctl, &s_item, N, G, tiles, it)) {
-    const size_t sbase = (size_t)it.n * sample_vecs * 16;
-    const char* xs = reinterpret_cast<const char*>(x) + sbase;
-    const char* ds = reinterpret_cast<const char*>(dy) + sbase;
-    const uint32_t v0 = (uint32_t)it.t * TH * ITER + threadIdx.x;
-    // ReLU-gate constants of this sample's channels
-    float sa[PACKED ? 1 : V], sbv[PACKED ? 1 : V];
-    uint32_t thr[V / 2 > 0 ? V / 2 : 1];
-    {
-      float sa_[V], sb_[V];
-#pragma unroll
-      for (int i = 0; i < V; ++i) {
-        const int c = tcol * V + i, g = c / cpg;
-        const float mean = stats[((size_t)it.n * GN_GROUPS + g) * 2 + 0], rstd = stats[((size_t)it.n * GN_GROUPS + g) * 2 + 1];
-        sa_[i] = rstd * gamma[c];
-        sb_[i] = beta[c] - mean * sa_[i];
-      }
-      if (PACKED) {
-#pragma unroll
-        for (int i = 0; i < V / 2; ++i)
-          thr[i] = gn2::floor_bf16_bits(-sb_[2 * i] / sa_[2 * i]) | (gn2::floor_bf16_bits(-sb_[2 * i + 1] / sa_[2 * i + 1]) << 16);
-      } else {
-#pragma unroll
-        for (int i = 0; i < V; ++i) { sa[PACKED ? 0 : i] = sa_[i]; sbv[PACKED ? 0 : i] = sb_[i]; }
-      }
-    }
-    auto gate = [&](const uint4& vx, const uint4& vd, float* fx, float* fd) {
-      A::unpack(vx, fx);
-      if (PACKED) {
-        uint4 m;
-        m.x = vd.x & gn2::gt2_mask(vx.x, thr[0]); m.y = vd.y & gn2::gt2_mask(vx.y, thr[1]);
-        m.z = vd.z & gn2::gt2_mask(vx.z, thr[V / 2 > 2 ? 2 : 0]); m.w = vd.w & gn2::gt2_mask(vx.w, thr[V / 2 > 3 ? 3 : 0]);
-        A::unpack(m, fd);
-      } else {
-        A::unpack(vd, fd);
-#pragma unroll
-        for (int i = 0; i < V; ++i) fd[i] = fmaf(sa[PACKED ? 0 : i], fx[i], sbv[PACKED ? 0 : i]) > 0.f ? fd[i] : 0.f;
-      }
-    };
-    if (it.phase == 0) {
-      float a[V], bq[V];
-#pragma unroll
-      for (int i = 0; i < V; ++i) { a[i] = 0.f; bq[i] = 0.f; }
-#pragma unroll
-      for (int j0 = 0; j0 < ITER; j0 += UB) {
-        uint4 vx[UB], vd[UB];
-#pragma unroll
-        for (int j = 0; j < UB; ++j) {
-          const uint32_t vi = v0 + (j0 + j) * TH;
-          const bool in = vi < sample_vecs;
-          vx[j] = in ? gn2::ldg128(xs + (size_t)vi * 16) : make_uint4(0u, 0u, 0u, 0u);
-          vd[j] = in ? gn2::ldg128(ds + (size_t)vi * 16) : make_uint4(0u, 0u, 0u, 0u);
-        }
-#pragma unroll
-        for (int j = 0; j < UB; ++j) {
-          float fx[V], fd[V]; gate(vx[j], vd[j], fx, fd);
-#pragma unroll
-          for (int i = 0; i < V; ++i) { a[i] += fd[i]; bq[i] = fmaf(fd[i], fx[i], bq[i]); }
-        }
-      }
-#pragma unroll
-      for (int i = 0; i < V; ++i) {
-        const int c = tcol * V + i, g = c / cpg;
-        const float mean = stats[((size_t)it.n * GN_GROUPS + g) * 2 + 0], rstd = stats[((size_t)it.n * GN_GROUPS + g) * 2 + 1];
-        const float ga = gamma[c], A_ = a[i];
-        a[i] = ga * A_;
-        bq[i] = rstd * ga * (bq[i] - mean * A_);
-      }
-      publish<V>(a, bq, C, tp, part, partial, ctl, N, it.n, it.t, tiles, &s_flag, m12,
-                 [&](float s, float q, float& o0, float& o1) { o0 = s * inv_m; o1 = q * inv_m; });
-    } else {
-      wait_ready(ctl, N, it.n);
-      float k1[V], k2[V], k3[V];
-#pragma unroll
-      for (int i = 0; i < V; ++i) {
-        const int c = tcol * V + i, g = c / cpg;
-        const float mean = stats[((size_t)it.n * GN_GROUPS + g) * 2 + 0], rstd = stats[((size_t)it.n * GN_GROUPS + g) * 2 + 1];
-        const float m1 = __ldcg(m12 + ((size_t)it.n * GN_GROUPS + g) * 2), m2 = __ldcg(m12 + ((size_t)it.n * GN_GROUPS + g) * 2 + 1);
-        k1[i] = rstd * gamma[c];
-        k2[i] = -rstd * rstd * m2;
-        k3[i] = -rstd * m1 - k2[i] * mean;
-      }
-      char* os = reinterpret_cast<char*>(dx) + sbase;
-      const char* as = addend ? reinterpret_cast<const char*>(addend) + sbase : nullptr;
-      const bool has_add = as != nullptr;
-#pragma unroll
-      for (int j0 = 0; j0 < ITER; j0 += UB) {
-        uint4 vx[UB], vd[UB], va[UB];
-#pragma unroll
-        for (int j = 0; j < UB; ++j) {
-          const uint32_t vi = v0 + (j0 + j) * TH;
-          const bool in = vi < sample_vecs;
-          vx[j] = in ? gn2::ldg128(xs + (size_t)vi * 16) : make_uint4(0u, 0u, 0u, 0u);
-          vd[j] = in ? gn2::ldg128(ds + (size_t)vi * 16) : make_uint4(0u, 0u, 0u, 0u);
-          if (has_add) va[j] = in ? gn2::ldg128(as + (size_t)vi * 16) : make_uint4(0u, 0u, 0u, 0u);
-        }
-#pragma unroll
-        for (int j = 0; j < UB; ++j) {
-          const uint32_t vi = v0 + (j0 + j) * TH;
-          float fx[V], fd[V], fo[V];
-          gate(vx[j], vd[j], fx, fd);
-          if (has_add) A::unpack(va[j], fo);
-#pragma unroll
-          for (int i = 0; i < V; ++i) {
-            const float tt = fmaf(k1[i], fd[i], fmaf(k2[i], fx[i], k3[i]));
-            fo[i] = has_add ? fo[i] + tt : tt;
-          }
-          if (vi < sample_vecs) *reinterpret_cast<uint4*>(os + (size_t)vi * 16) = A::pack(fo);
-        }
-      }
-    }
-  }
-}
-}  // namespace gn3
-
 void gn2_set_trace(unsigned long long* dev_ptr) { cudaMemcpyToSymbol(gn2::g_trace, &dev_ptr, sizeof(dev_ptr)); }
 
-static int g_gn_version = -1;   // DORPATCH_GN: v2 (default, cluster per sample), v3 (streaming two-phase; measured slower), v1, twopass
-static int gn_version() {
-  if (g_gn_version < 0) {
-    const char* e = getenv("DORPATCH_GN");
-    g_gn_version = (e && strcmp(e, "v1") == 0) ? 1 : ((e && strcmp(e, "twopass") == 0) ? 0 : ((e && strcmp(e, "v3") == 0) ? 3 : 2));
-  }
-  return g_gn_version;
-}
-static int gn2_env(const char* name, int dflt) { const char* e = getenv(name); return e ? atoi(e) : dflt; }
-static int gn2_max_cluster() {
-  static int v = -1;
-  if (v < 0) v = gn2_env("DORPATCH_GN2_MAXCL", 16);
-  return v;
-}
+// v2 plan limits, chosen by the round-2 sweeps (tools/r2_batch2.sh, r2_batch14.sh): the largest cluster (16 needs the
+// non-portable size), the shared memory per CTA that still fits two CTAs per SM, the most one CTA may take, and whether a
+// backward CTA that has an SM to itself also keeps its dy slab in shared memory
+constexpr int GN2_MAX_CLUSTER = 16;
+constexpr size_t GN2_SOFT = 111 * 1024, GN2_HARD = 224 * 1024;
+constexpr bool GN2_DYS_BIG = true;
 // forward: smallest cluster whose slab leaves room for two CTAs per SM (256 threads), else one 512-thread CTA per SM
 static bool gn2_plan_fwd(int P, int C, size_t es, gn2::Plan* pl) {
-  static const size_t soft = (size_t)gn2_env("DORPATCH_GN2_SOFT", 111) * 1024, hard = 224 * 1024;
   const int V = (int)(16 / es);
   if (C % (V * 1) != 0 || (C / V) > 256 || 256 % (C / V) != 0) return false;
-  const size_t f256 = gnc::HDR + gnc::tp_bytes(256), f512 = gnc::HDR + gnc::tp_bytes(512);
-  for (int cl = 1; cl <= gn2_max_cluster(); cl *= 2) {
+  const size_t f256 = gn2::HDR + gn2::tp_bytes(256), f512 = gn2::HDR + gn2::tp_bytes(512);
+  for (int cl = 1; cl <= GN2_MAX_CLUSTER; cl *= 2) {
     if (cl > P) break;
     const size_t slab = (((size_t)((P + cl - 1) / cl)) * C * es + 127) / 128 * 128;
     if (slab > gn2::MAX_CHUNKS * (size_t)gn2::CHUNK) continue;
-    if (f256 + slab <= soft) { *pl = gn2::Plan{cl, 256, false, f256 + slab, (uint32_t)slab}; return true; }
+    if (f256 + slab <= GN2_SOFT) { *pl = gn2::Plan{cl, 256, false, f256 + slab, (uint32_t)slab}; return true; }
   }
-  for (int cl = 1; cl <= gn2_max_cluster(); cl *= 2) {
+  for (int cl = 1; cl <= GN2_MAX_CLUSTER; cl *= 2) {
     if (cl > P) break;
     const size_t slab = (((size_t)((P + cl - 1) / cl)) * C * es + 127) / 128 * 128;
     if (slab > gn2::MAX_CHUNKS * (size_t)gn2::CHUNK) continue;
-    if (f512 + slab <= hard && 512 % (C / V) == 0) { *pl = gn2::Plan{cl, 512, false, f512 + slab, (uint32_t)slab}; return true; }
+    if (f512 + slab <= GN2_HARD && 512 % (C / V) == 0) { *pl = gn2::Plan{cl, 512, false, f512 + slab, (uint32_t)slab}; return true; }
   }
   return false;
 }
 // backward: both slabs resident when they fit (two CTAs per SM, else one), else x resident + dy streamed
 static bool gn2_plan_bwd(int P, int C, size_t es, gn2::Plan* pl) {
-  static const size_t soft = (size_t)gn2_env("DORPATCH_GN2_SOFT", 111) * 1024, hard = 224 * 1024;
-  static const int dys_big = gn2_env("DORPATCH_GN2_DYS_BIG", 1);
   const int V = (int)(16 / es);
   if ((C / V) > 256 || 256 % (C / V) != 0) return false;
-  const size_t f256 = gnc::HDR + gnc::tp_bytes(256), f512 = gnc::HDR + gnc::tp_bytes(512);
-  for (int cl = 1; cl <= gn2_max_cluster(); cl *= 2) {
+  const size_t f256 = gn2::HDR + gn2::tp_bytes(256), f512 = gn2::HDR + gn2::tp_bytes(512);
+  for (int cl = 1; cl <= GN2_MAX_CLUSTER; cl *= 2) {
     if (cl > P) break;
     const size_t slab = (((size_t)((P + cl - 1) / cl)) * C * es + 127) / 128 * 128;
-    if (f256 + 2 * slab <= soft) { *pl = gn2::Plan{cl, 256, true, f256 + 2 * slab, (uint32_t)slab}; return true; }
+    if (f256 + 2 * slab <= GN2_SOFT) { *pl = gn2::Plan{cl, 256, true, f256 + 2 * slab, (uint32_t)slab}; return true; }
   }
-  if (dys_big)
-    for (int cl = 1; cl <= gn2_max_cluster(); cl *= 2) {
+  if (GN2_DYS_BIG)
+    for (int cl = 1; cl <= GN2_MAX_CLUSTER; cl *= 2) {
       if (cl > P) break;
       const size_t slab = (((size_t)((P + cl - 1) / cl)) * C * es + 127) / 128 * 128;
-      if (f512 + 2 * slab <= hard && 512 % (C / V) == 0) { *pl = gn2::Plan{cl, 512, true, f512 + 2 * slab, (uint32_t)slab}; return true; }
+      if (f512 + 2 * slab <= GN2_HARD && 512 % (C / V) == 0) { *pl = gn2::Plan{cl, 512, true, f512 + 2 * slab, (uint32_t)slab}; return true; }
     }
   gn2::Plan f;
   if (!gn2_plan_fwd(P, C, es, &f)) return false;
   *pl = f;
   pl->dys = false;
   return true;
-}
-
-static int gn3_group(size_t sample_bytes, int streams, int N) {
-  static const size_t l2mb = (size_t)gn2_env("DORPATCH_GN3_L2MB", 24);
-  size_t g = (l2mb << 20) / (sample_bytes * (size_t)streams);
-  if (g < 1) g = 1;
-  if (g > (size_t)N) g = (size_t)N;
-  return (int)g;
-}
-template <typename K>
-static int gn3_grid(K kernel, int total_items) {
-  static std::map<const void*, int> cache;
-  const void* key = (const void*)kernel;
-  auto it = cache.find(key);
-  int per_sm;
-  if (it == cache.end()) {
-    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, gn3::TH, 0) != cudaSuccess || per_sm < 1) { cudaGetLastError(); per_sm = 1; }
-    cache[key] = per_sm;
-  } else per_sm = it->second;
-  if (g_num_sms == 0) { int dev = 0; cudaGetDevice(&dev); cudaDeviceGetAttribute(&g_num_sms, cudaDevAttrMultiProcessorCount, dev); }
-  const int cap = g_num_sms * per_sm;
-  return total_items < cap ? total_items : cap;
-}
-// workspace (floats): partial [N][tiles][64] | m12 [N][64] | ctl (uint32) [32 + 2N]
-static bool gn3_workspace(float* ws, int N, int tiles, float** partial, float** m12, unsigned** ctl) {
-  if ((size_t)N * tiles * 64 + (size_t)N * 64 + 32 + 2 * (size_t)N > (size_t)N * GN_WS_FLOATS_PER_SAMPLE + GN_WS_FLOATS_EXTRA) return false;
-  *partial = ws;
-  *m12 = ws + (size_t)N * tiles * 64;
-  *ctl = reinterpret_cast<unsigned*>(*m12 + (size_t)N * 64);
-  return true;
-}
-static bool launch_gn3_forward(const void* x, void* y, const float* gamma, const float* beta, float* ws, float* stats, int N, int P,
-                               int C, bool bf16, cudaStream_t st) {
-  const size_t es = bf16 ? 2 : 4;
-  const int V = (int)(16 / es), cols = C / V;
-  if (ws == nullptr || cols > gn3::TH || gn3::TH % cols != 0) return false;
-  static const int iter = gn2_env("DORPATCH_GN3_ITER", 16);
-  const int ITER = iter == 8 ? 8 : 16;
-  const size_t sample_vecs = (size_t)P * cols;
-  const int tiles = (int)((sample_vecs + (size_t)gn3::TH * ITER - 1) / ((size_t)gn3::TH * ITER));
-  float *partial, *m12; unsigned* ctl;
-  if (!gn3_workspace(ws, N, tiles, &partial, &m12, &ctl)) return false;
-  const int G = gn3_group(sample_vecs * 16, 1, N);
-  cudaMemsetAsync(ctl, 0, (size_t)(gn3::CTL_WORDS + 2 * N) * 4, st);
-  const int total = 2 * N * tiles;
-#define GN3F(TT, IT) gn3::fwd_kernel<TT, IT><<<gn3_grid(gn3::fwd_kernel<TT, IT>, total), gn3::TH, 0, st>>>((const TT*)x, (TT*)y, gamma, beta, stats, partial, ctl, N, P, C, G, tiles)
-  if (bf16) { if (ITER == 8) GN3F(__nv_bfloat16, 8); else GN3F(__nv_bfloat16, 16); }
-  else { if (ITER == 8) GN3F(float, 8); else GN3F(float, 16); }
-#undef GN3F
-  return cudaPeekAtLastError() == cudaSuccess;
-}
-static bool launch_gn3_backward(const void* dy, const void* x, const void* addend, void* dx, const float* gamma, const float* beta,
-                                const float* stats, float* ws, int N, int P, int C, bool bf16, bool gamma_pos, cudaStream_t st) {
-  const size_t es = bf16 ? 2 : 4;
-  const int V = (int)(16 / es), cols = C / V;
-  if (ws == nullptr || cols > gn3::TH || gn3::TH % cols != 0) return false;
-  constexpr int ITER = 8;
-  const size_t sample_vecs = (size_t)P * cols;
-  const int tiles = (int)((sample_vecs + (size_t)gn3::TH * ITER - 1) / ((size_t)gn3::TH * ITER));
-  float *partial, *m12; unsigned* ctl;
-  if (!gn3_workspace(ws, N, tiles, &partial, &m12, &ctl)) return false;
-  const int G = gn3_group(sample_vecs * 16, 2, N);
-  cudaMemsetAsync(ctl, 0, (size_t)(gn3::CTL_WORDS + 2 * N) * 4, st);
-  const int total = 2 * N * tiles;
-  const bool neg = bf16 ? !gamma_pos : true;
-#define GN3B(TT, NEG) gn3::bwd_kernel<TT, ITER, NEG><<<gn3_grid(gn3::bwd_kernel<TT, ITER, NEG>, total), gn3::TH, 0, st>>>((const TT*)dy, (const TT*)x, (const TT*)addend, (TT*)dx, gamma, beta, stats, partial, m12, ctl, N, P, C, G, tiles)
-  if (bf16) { if (neg) GN3B(__nv_bfloat16, true); else GN3B(__nv_bfloat16, false); }
-  else GN3B(float, true);
-#undef GN3B
-  return cudaPeekAtLastError() == cudaSuccess;
 }
 
 static bool launch_gn2_forward(const void* x, void* y, const float* gamma, const float* beta, float* stats, int N, int P,
@@ -2143,58 +1213,14 @@ static bool launch_gn2_backward(const void* dy, const void* x, const void* adden
 
 void launch_gn_relu_forward(const void* x, void* y, const float* gamma, const float* beta, float* partial,
                             float* stats, int N, int P, int C, bool bf16, cudaStream_t st) {
-  if (gn_version() == 3 && launch_gn3_forward(x, y, gamma, beta, partial, stats, N, P, C, bf16, st)) return;
-  if (gn_version() >= 2 && launch_gn2_forward(x, y, gamma, beta, stats, N, P, C, bf16, st)) return;
-  GnPlan pl;
-  if (gn_version() >= 1 && gn_plan(P, C, bf16 ? 2 : 4, &pl)) {
-    const int grid = gn_grid(pl, N);
-    bool ok;
-    if (bf16) ok = launch_cluster(gn_fwd_cluster_kernel<__nv_bfloat16>, pl.cl, grid, pl.threads, pl.smem, st, (const __nv_bfloat16*)x, (__nv_bfloat16*)y, gamma, beta, stats, N, P, C, gn_nbuf(pl), pl.slab_stride);
-    else ok = launch_cluster(gn_fwd_cluster_kernel<float>, pl.cl, grid, pl.threads, pl.smem, st, (const float*)x, (float*)y, gamma, beta, stats, N, P, C, gn_nbuf(pl), pl.slab_stride);
-    if (ok) return;
-    cudaGetLastError();   // clear and fall back
-  }
+  if (launch_gn2_forward(x, y, gamma, beta, stats, N, P, C, bf16, st)) return;
   launch_gn_relu_forward_2pass(x, y, gamma, beta, partial, stats, N, P, C, bf16, st);
 }
 
 void launch_gn_relu_backward(const void* dy, const void* x, const void* addend, void* dx, const float* gamma,
                              const float* beta, const float* stats, float* partial, int N, int P, int C, bool bf16,
                              cudaStream_t st, bool gamma_pos) {
-  if (gn_version() == 3 && launch_gn3_backward(dy, x, addend, dx, gamma, beta, stats, partial, N, P, C, bf16, gamma_pos, st)) return;
-  if (gn_version() >= 2 && launch_gn2_backward(dy, x, addend, dx, gamma, beta, stats, N, P, C, bf16, gamma_pos, st)) return;
-  GnPlan pl;
-  const bool ug = (C / GN_GROUPS) >= (bf16 ? 8 : 4);
-  if (gn_version() >= 1) {   // both slabs in shared memory when they fit (DORPATCH_GN_DYSMEM=0 disables)
-    static int dys = -1;
-    if (dys < 0) { const char* e = getenv("DORPATCH_GN_DYSMEM"); dys = e ? atoi(e) : 1; }
-    const size_t es = bf16 ? 2 : 4, fixed = gnc::HDR + gnc::tp_bytes(gnc::THREADS);
-    if (dys && gn_plan(P, C, es, &pl) && !pl.persistent && C / (int)(16 / es) <= gnc::THREADS) {
-      for (int cl = 1; cl <= 8; cl *= 2) {
-        if (cl > P) break;
-        const size_t slab = (((size_t)((P + cl - 1) / cl)) * C * es + 127) / 128 * 128;
-        if (fixed + 2 * slab <= 111 * 1024) {
-          bool ok;
-#define GNS(TT, UGV) launch_cluster(gn_bwd_cluster_smem_kernel<TT, UGV>, cl, cl * N, gnc::THREADS, fixed + 2 * slab, st, (const TT*)dy, (const TT*)x, (const TT*)addend, (TT*)dx, gamma, beta, stats, P, C, (uint32_t)slab)
-          if (bf16) ok = ug ? GNS(__nv_bfloat16, true) : GNS(__nv_bfloat16, false);
-          else ok = ug ? GNS(float, true) : GNS(float, false);
-#undef GNS
-          if (ok) return;
-          cudaGetLastError();
-          break;
-        }
-      }
-    }
-  }
-  if (gn_version() >= 1 && gn_plan(P, C, bf16 ? 2 : 4, &pl)) {
-    const int grid = gn_grid(pl, N);
-    bool ok;
-#define GNB(TT, UGV) launch_cluster(gn_bwd_cluster_kernel<TT, UGV>, pl.cl, grid, pl.threads, pl.smem, st, (const TT*)dy, (const TT*)x, (const TT*)addend, (TT*)dx, gamma, beta, stats, N, P, C, gn_nbuf(pl), pl.slab_stride)
-    if (bf16) ok = ug ? GNB(__nv_bfloat16, true) : GNB(__nv_bfloat16, false);
-    else ok = ug ? GNB(float, true) : GNB(float, false);
-#undef GNB
-    if (ok) return;
-    cudaGetLastError();
-  }
+  if (launch_gn2_backward(dy, x, addend, dx, gamma, beta, stats, N, P, C, bf16, gamma_pos, st)) return;
   launch_gn_relu_backward_2pass(dy, x, addend, dx, gamma, beta, stats, partial, N, P, C, bf16, st);
 }
 
@@ -2202,12 +1228,12 @@ void launch_gn_stats(const void* x, float* partial, float* stats, int N, int P, 
   const int V = bf16 ? 8 : 4, cols = C / V;
   const size_t nvec = (size_t)P * cols;
   const int tiles = (int)((nvec + gn2::ST_TILE - 1) / gn2::ST_TILE);
-  if (gn_version() >= 2 && cols <= gn2::ST_TH && gn2::ST_TH % cols == 0 && C % V == 0 && tiles * 64 <= GN_WS_FLOATS_PER_SAMPLE) {
+  if (cols <= gn2::ST_TH && gn2::ST_TH % cols == 0 && C % V == 0 && tiles * 64 <= GN_WS_FLOATS_PER_SAMPLE) {
     DISPATCH_T(bf16, (gn2::stats_kernel<T><<<dim3(tiles, N), gn2::ST_TH, 0, st>>>((const T*)x, partial, P, C, tiles)));
     DISPATCH_T(bf16, (gn_finalize_kernel<T><<<N, 32, 0, st>>>(partial, stats, P, C, tiles)));
     return;
   }
-  launch_gn_stats_v1(x, partial, stats, N, P, C, bf16, st);
+  launch_gn_stats_2pass(x, partial, stats, N, P, C, bf16, st);
 }
 
 }  // namespace dp

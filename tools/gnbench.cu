@@ -3,7 +3,7 @@
 // restatement of timm's GroupNormAct (torch.nn.functional.group_norm + relu, eps 1e-5) and its input gradient.
 //   nvcc -O3 -std=c++17 -gencode arch=compute_100a,code=sm_100a -o gnbench tools/gnbench.cu \
 //        -Ldorpatch_b200/lib -ldorpatch -Xlinker -rpath,$PWD/dorpatch_b200/lib
-//   DORPATCH_GN=v1|v2 ./gnbench [N] [only_C]
+//   ./gnbench [N] [only_C]
 // Buffers rotate over > 300 MB so that no launch finds its operands in the 126 MB L2.
 #include <cuda_bf16.h>
 #include <cuda_runtime.h>
